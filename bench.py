@@ -2,6 +2,7 @@
 """bench.py — NCMC steps/s on the T4 lysozyme L99A – toluene workload (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--replicas R] [--workload NAME] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path — one NCMC integrator step (H V R O R V H with work accumulation) of every
 walker held by the GPU.  N > 1 is launched by torchrun, one rank per GPU; walkers are independent (weak scaling,
@@ -19,6 +20,8 @@ Printed JSON (one line, rank 0):
   cpu_baseline the oracle's C twin (reference semantics, all host cores) on a bounded sample; `cpu_optimised` the same
                code with one force evaluation per step (the lambda-separable trick the engine uses), for context
   m3           BASELINE configs[2]: 64 walkers in total, 64 / N per GPU (same timed region)
+`--dump-outputs DIR` also writes what the timed path computed in its last step as DIR/<name>.npy (see dump_outputs), so
+that two builds can be compared output for output on identical inputs.
 `--impl reference` times the CPU implementation alone (the reference stack — OpenMM/openmmtools/parmed — is not
 installable here; rank 0 only, all host cores whatever OMP_NUM_THREADS the launcher exported).
 """
@@ -38,6 +41,7 @@ sys.path.insert(0, ROOT)
 FLOP_PER_PAIR = 60            # SURVEY.md §8(d)
 FP32_PEAK_NOMINAL_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12
 SEED = 20261017
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def host_cores():
@@ -57,11 +61,17 @@ def make_config(wl, replicas, world):
 
 
 def protocol_warmup(W, K, nsteps_nc):
-    """Warm-up and window length actually used: short protocols (M1) keep the timed region inside one protocol."""
+    """Warm-up and window length actually used: a window must fit inside one protocol after the warm-up, so short
+    protocols (M1) shorten the warm-up and, without --steps (K None), the window; a K given is never changed, and one
+    that cannot fit is an error."""
     W = max(W, 3)
-    if K + W >= nsteps_nc:
+    if (K or 1000) + W >= nsteps_nc:
         W = min(W, max(3, nsteps_nc // 5))
-        K = nsteps_nc - W - 2
+    if K is None:
+        K = min(1000, nsteps_nc - W - 2)
+    if K < 1 or K + W + 2 > nsteps_nc:
+        raise SystemExit('bench: --steps %d does not fit in one %d-step protocol after %d warm-up steps (1 to %d)'
+                         % (K, nsteps_nc, W, nsteps_nc - W - 2))
     return W, K
 
 
@@ -148,6 +158,31 @@ class ClockSampler(object):
                 'source': 'nvml (in-process)' if self._nvml is not None else 'nvidia-smi'}
 
 
+def dump_outputs(out_dir, ctx, integ, n_atoms, n_rep):
+    """What a caller of the timed path receives after its last step, as <out_dir>/<name>.npy in float64: positions (nm),
+    velocities (nm/ps) and forces (kJ/mol/nm) of every walker as (walker, atom, xyz), and per walker the potential and
+    kinetic energy (kJ/mol) and the protocol work (kT).  Where that would exceed 64 MB, the same fixed, seeded sample of
+    atoms is kept in every run and its indices are written as atom_index.npy."""
+    eng = ctx._engine
+    atoms = slice(None)
+    per_atom = 3 * 3 * 8 * n_rep + 8
+    budget = DUMP_LIMIT_BYTES - 3 * 8 * n_rep - 4096           # less the per-walker scalars and the .npy headers
+    if per_atom * n_atoms > budget:
+        keep = budget // per_atom
+        atoms = np.sort(np.random.default_rng(SEED).choice(n_atoms, keep, replace=False))
+    ep, ek = eng.get_energy()
+    out = {'positions': [eng.get_positions(r)[atoms] for r in range(n_rep)],
+           'velocities': [eng.get_velocities(r)[atoms] for r in range(n_rep)],
+           'forces': [eng.get_forces(r)[atoms] for r in range(n_rep)],
+           'potential_energy': ep, 'kinetic_energy': ek,
+           'protocol_work': [integ.get_protocol_work(dimensionless=True, replica=r) for r in range(n_rep)]}
+    if not isinstance(atoms, slice):
+        out['atom_index'] = atoms
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), np.asarray(a, dtype=np.float64))
+
+
 def cpu_relax(topo, x, iters=60, max_disp=0.005):
     """Capped steepest descent with the constraints re-imposed (CPU oracle): the TOL-parm start coordinates carry
     the type-index quirk documented in DESIGN.md §8 and, like the reference's tests, need minimising before dynamics."""
@@ -232,7 +267,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=1000)
+    ap.add_argument('--steps', type=int, default=None,
+                    help='timed steps per window (default 1000, or as many as fit in a shorter protocol)')
     ap.add_argument('--warmup', type=int, default=200)
     ap.add_argument('--windows', type=int, default=20, help='timed windows of K steps per rank (median reported)')
     ap.add_argument('--replicas', type=int, default=0, help='independent walkers per GPU (0 = the workload\'s own)')
@@ -243,6 +279,8 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--batched', type=int, default=8, help='also report a batched run with this many walkers (0 = skip)')
     ap.add_argument('--m3-walkers', type=int, default=64, help='BASELINE configs[2]: total walkers of the m3 block (0 = skip)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the timed path computed in its last step as DIR/<name>.npy (rank 0\'s walkers)')
     args = ap.parse_args()
     if args.impl == 'reference':
         return run_reference(args)
@@ -543,6 +581,23 @@ def main():
         except Exception as err:
             cpu_opt = {'unavailable': str(err)}
 
+    # ---- outputs of the timed path ------------------------------------------------------------------------------------
+    dump = None
+    if args.dump_outputs:
+        # The timed windows are not reproducible step for step: the clock warm-up and the window budget are wall-clock
+        # bounded, and the thermostat's noise stream runs on across protocol restarts.  So the timed path is run once more
+        # on a fresh context with the timed run's seed and start (minimised coordinates, velocities drawn at 300 K, the
+        # same W warm-up steps, one window of K steps) and the state after its last step is written: an equivalent run
+        # with identical inputs in every run, not a copy of the last timed window.  A blown-up walker leaves NaN in the
+        # files and ok = false in the JSON line.
+        ctx_d, integ_d = make_context(R, SEED + 1000 * rank)
+        ok = step_or_flag(integ_d, W) and step_or_flag(integ_d, K)
+        dump_outputs(args.dump_outputs, ctx_d, integ_d, topo['n_atoms'], R)
+        dump = {'dir': args.dump_outputs, 'warmup': W, 'steps': K, 'replicas': R, 'ok': bool(ok),
+                'what': 'state after the last of K steps of a fresh context with the timed run\'s seed and start, after W '
+                        'warm-up steps'}
+        del ctx_d, integ_d
+
     line = {'metric': 'NCMC steps/s (aggregate)', 'value': value, 'unit': 'steps/s', 'n_gpus': world, 'steps': K,
             'warmup': W, 'ms_per_step': ms_max / K, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
             'dtype': 'f32 pair math / f64 integration / i64 fixed-point accumulation', 'data': 'synthetic',
@@ -559,7 +614,7 @@ def main():
             'gpu_launches': int(launches), 'clocks': clocks.summary(), 'roofline': roofline, 'roofline_hbm': roofline_hbm,
             'kernels_us_per_step': {k: round(v['us_per_step'], 2) for k, v in ktimes.items()},
             'cpu_baseline': cpu, 'cpu_optimised': cpu_opt, 'batched': batched, 'm3': m3,
-            'blown_up_walkers': nan_events[0],
+            'blown_up_walkers': nan_events[0], 'dump': dump,
             'walker_stats': {'n': int(len(stats)), 'mean_work_kT': float(np.nanmean(stats[:, 0])),
                              'accepted': int(stats[:, 1].sum())}}
     print(json.dumps(line))

@@ -1,8 +1,8 @@
 """Generate the committed fixtures under tests/golden/ from the reference's data files.
 
-Run in the build container (``/root/reference`` is absent on the GPU box):
+Run with ``BLUES_REFERENCE_DATA`` naming ``blues/tests/data`` of a MobleyLab/blues checkout:
 
-    python tests/golden/make_fixtures.py
+    BLUES_REFERENCE_DATA=<checkout>/blues/tests/data python tests/golden/make_fixtures.py [--reference-tests | --spread-lambda]
 
 Outputs
   tol_parm.npz / wat_divaline.npz / vac_divaline.npz
@@ -16,6 +16,9 @@ Outputs
       constraint topology and PME grid — NOT a physical model of T4L.
   oracle_vectors.npz
       Energies (by term) and forces of the float64 oracle on those systems, for the CPU-side golden tests.
+  spread_lambda_protocol.json (--spread-lambda)
+      utils.spreadLambdaProtocol tables for the cases of tests/test_host_logic.py; its ``source`` entry says which
+      function computed them (the reference's, executed from its source text, or this package's).
 """
 import os
 import sys
@@ -25,7 +28,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = os.environ.get('BLUES_REFERENCE_DATA', '/root/reference/blues/tests/data')
+REF = os.environ.get('BLUES_REFERENCE_DATA')
 
 from blues_b200.structure import Structure, load_file, load_pdb, read_inpcrd  # noqa: E402
 from blues_b200 import unit as u  # noqa: E402
@@ -412,10 +415,51 @@ def reference_tests():
         shutil.copyfile(os.path.join(root, 'tests', name), os.path.join(dst, name))
     for name in ('TOL-parm.prmtop', 'TOL-parm.inpcrd', 'ethylene_system.xml', 'ethylene_structure.pdb'):
         shutil.copyfile(os.path.join(REF, name), os.path.join(dst, 'data', name))
+    import hashlib
+    digests = {}
+    for rel in ('test_simulation.py', 'test_randomrotation.py', 'test_ethylene.py', 'data/TOL-parm.prmtop',
+                'data/TOL-parm.inpcrd', 'data/ethylene_system.xml', 'data/ethylene_structure.pdb'):
+        with open(os.path.join(dst, rel), 'rb') as fh:
+            digests[rel] = hashlib.sha256(fh.read()).hexdigest()
+    with open(os.path.join(HERE, 'reference_checkout_sha256.json'), 'w') as fh:
+        json.dump(digests, fh, indent=1, sort_keys=True)
+        fh.write('\n')
     print('reference test fixtures refreshed under', dst)
 
 
+def spread_lambda_fixture():
+    """spreadLambdaProtocol (blues/utils.py:276-369) for the schedules and step counts tests/test_host_logic.py checks →
+    spread_lambda_protocol.json.  With BLUES_REFERENCE_DATA set the reference's function runs from its source text;
+    without it, this package's utils.spreadLambdaProtocol does, and ``source`` records which."""
+    import ast
+    import json
+    from scipy.interpolate import interp1d
+    from tests.test_host_logic import SPREAD_LAMBDA_CASES
+    if REF:
+        path = os.path.join(os.path.dirname(os.path.dirname(REF)), 'utils.py')
+        tree = ast.parse(open(path).read())
+        fn = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == 'spreadLambdaProtocol'][0]
+        ns = {'np': np, 'interp1d': interp1d, 'floor': math.floor}
+        exec(compile(ast.Module([fn], []), path, 'exec'), ns)
+        spread, source = ns['spreadLambdaProtocol'], 'reference blues/utils.py spreadLambdaProtocol'
+    else:
+        from blues_b200 import utils
+        spread, source = utils.spreadLambdaProtocol, 'blues_b200.utils.spreadLambdaProtocol'
+    out = {'source': source, 'tables': {}}
+    for name, vals, kind, n in SPREAD_LAMBDA_CASES:
+        out['tables']['%s/%s/%d' % (name, kind, n)] = [float(v) for v in spread(list(vals), n, switching_types=kind,
+                                                                                 return_tab_function=False)]
+    with open(os.path.join(HERE, 'spread_lambda_protocol.json'), 'w') as f:
+        json.dump(out, f)
+        f.write('\n')
+    print('spreadLambdaProtocol tables:', len(out['tables']), 'from', source)
+
+
 def main():
+    if '--spread-lambda' in sys.argv:
+        return spread_lambda_fixture()
+    if not REF:
+        raise SystemExit('set BLUES_REFERENCE_DATA to <MobleyLab/blues checkout>/blues/tests/data')
     if '--reference-tests' in sys.argv:
         return reference_tests()
     reference_bookkeeping()

@@ -30,7 +30,7 @@ compat.install(data_root=%(ref)r)
 import blues_b200._native as native
 assert native.Engine.__module__ == 'blues_b200._native'      # the real engine class, not a stand-in
 import pytest
-rc = pytest.main(['-p', 'no:cacheprovider', '-q', '-rA', '--tb=short', '--rootdir', %(tmp)r, '-c', '/dev/null', %(tmp)r])
+rc = pytest.main(['-p', 'no:cacheprovider', '-q', '-rA', '--tb=short', '--rootdir', %(tmp)r, '-c', '/dev/null', '--confcutdir', %(tmp)r, %(tmp)r])
 print('ENGINES_CREATED', native.Engine.created if hasattr(native.Engine, 'created') else -1)
 sys.exit(rc)
 '''

@@ -527,13 +527,19 @@ _STERICS = [1.0, 1.0, 1.0, 1.0, 1.0, 1.0, 1.0, 0.95, 0.8848447462380346, 0.84283
             0.31648339779024653, 0.2780498882483276, 0.2521302239477468, 0.23139484523965026, 0.18729812232625365,
             0.15427643961733822, 0.12153116162972155, 0.09632462702545555, 0.06463743549588846, 0.01463743549588846, 0.0]
 _STATICS = [1.0, 0.8519493439593149, 0.7142750443470669, 0.5385929179832776, 0.3891972949356391, 0.18820309596839535] + [0.0] * 26
+# (schedule name, schedule, switching_types, steps) compared with golden/spread_lambda_protocol.json
+SPREAD_LAMBDA_CASES = [(name, vals, kind, n) for name, vals, kind in (('sterics', _STERICS, 'sterics'),
+                                                                      ('statics', _STATICS, 'auto'),
+                                                                      ('statics', _STATICS, 'electrostatics'))
+                       for n in (100, 37, 1000)]
 
 
 def test_spread_lambda_protocol_and_tabulated_functions_in_the_integrator():
     """utils.spreadLambdaProtocol (blues/utils.py:276-369; the schedules are the ones of its docstring) and
     CustomIntegrator.addTabulatedFunction on the NCMC integrator: a symmetric protocol, plateaus exact, and the tables the
-    engine receives are the tabulated functions sampled at every lambda step.  Where the checkout is mounted the values
-    are compared with the reference's own function, executed from its source text (its module cannot be imported here)."""
+    engine receives are the tabulated functions sampled at every lambda step.  The values are compared with the tables
+    stored in golden/spread_lambda_protocol.json and, where ``BLUES_REFERENCE`` names a checkout, with the reference's own
+    function executed from its source text (its module cannot be imported here)."""
     import ast
     from blues_b200.lepton import Discrete1DFunction, Continuous1DFunction, Expression
     steps = 100
@@ -547,7 +553,13 @@ def test_spread_lambda_protocol_and_tabulated_functions_in_the_integrator():
     assert el[1] < 1.0 and st[9] == 1.0 and st[10] < 1.0                           # electrostatics go first
     with pytest.raises(ValueError):
         utils.spreadLambdaProtocol(_STATICS, steps, switching_types='bogus')
-    ref_src = os.path.join(os.environ.get('BLUES_REFERENCE', '/root/reference'), 'blues', 'utils.py')
+    with open(os.path.join(GOLDEN, 'spread_lambda_protocol.json')) as fh:
+        golden = json.load(fh)['tables']
+    assert sorted(golden) == sorted('%s/%s/%d' % (name, kind, n) for name, _, kind, n in SPREAD_LAMBDA_CASES)
+    for name, vals, kind, n in SPREAD_LAMBDA_CASES:
+        got = utils.spreadLambdaProtocol(list(vals), n, switching_types=kind, return_tab_function=False)
+        np.testing.assert_allclose(got, golden['%s/%s/%d' % (name, kind, n)], rtol=0, atol=1e-12)
+    ref_src = os.path.join(os.environ.get('BLUES_REFERENCE') or os.devnull, 'blues', 'utils.py')
     if os.path.exists(ref_src):
         tree = ast.parse(open(ref_src).read())
         fn = [n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == 'spreadLambdaProtocol'][0]
@@ -555,11 +567,10 @@ def test_spread_lambda_protocol_and_tabulated_functions_in_the_integrator():
         from scipy.interpolate import interp1d
         ns = {'np': np, 'interp1d': interp1d, 'floor': floor}
         exec(compile(ast.Module([fn], []), ref_src, 'exec'), ns)
-        for vals, kind in ((_STERICS, 'sterics'), (_STATICS, 'auto'), (_STATICS, 'electrostatics')):
-            for n in (100, 37, 1000):
-                want = ns['spreadLambdaProtocol'](list(vals), n, switching_types=kind, return_tab_function=False)
-                got = utils.spreadLambdaProtocol(list(vals), n, switching_types=kind, return_tab_function=False)
-                np.testing.assert_allclose(got, want, rtol=0, atol=1e-12)
+        for _, vals, kind, n in SPREAD_LAMBDA_CASES:
+            want = ns['spreadLambdaProtocol'](list(vals), n, switching_types=kind, return_tab_function=False)
+            got = utils.spreadLambdaProtocol(list(vals), n, switching_types=kind, return_tab_function=False)
+            np.testing.assert_allclose(got, want, rtol=0, atol=1e-12)
     # tabulated functions
     f = utils.spreadLambdaProtocol(_STERICS, steps, switching_types='sterics')
     assert isinstance(f, Discrete1DFunction) and f(0) == 1.0 and f(50.4) == f(50) and f(-1) == 0.0 and f(101) == 0.0

@@ -1,12 +1,15 @@
-"""The reference's own test file, unmodified, against this package through ``blues_b200.compat`` (SURVEY.md §8(f)2).
+"""The reference's own test files, unmodified, against this package through ``blues_b200.compat`` (SURVEY.md §8(f)2).
 
-Runs only where the reference checkout is mounted (this container: ``/root/reference``; it does not exist on the GPU
-box, and nothing is copied into the repository — the test file is copied to a temporary directory at run time because
-pytest would otherwise import it as ``blues.tests.…`` from the read-only checkout).  Without a GPU the host-side tests
-of ``blues/tests/test_simulation.py`` must pass as they are; every other test of that file must get as far as creating
-a ``Context`` and stop there with the engine's "no CUDA device … no CPU fallback" error — i.e. nothing is blocked by a
+The files come from the verbatim copies of MobleyLab/blues files under ``tests/golden/reference_checkout/`` (their
+SHA-256 digests are pinned in ``tests/golden/reference_checkout_sha256.json``), or from a checkout named by
+``BLUES_REFERENCE``.  The test file is copied to a temporary directory at run time because pytest would otherwise
+import it as ``blues.tests.…`` from the checkout.  Without a GPU the host-side tests of
+``blues/tests/test_simulation.py`` must pass as they are; every other test of that file must get as far as creating a
+``Context`` and stop there with the engine's "no CUDA device … no CPU fallback" error — i.e. nothing is blocked by a
 missing name or a different signature.
 """
+import hashlib
+import json
 import os
 import re
 import shutil
@@ -15,8 +18,9 @@ import sys
 
 import pytest
 
-REFERENCE = os.environ.get('BLUES_REFERENCE', '/root/reference')
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+CHECKOUT = os.path.join(ROOT, 'tests', 'golden', 'reference_checkout')
+REFERENCE = os.environ.get('BLUES_REFERENCE') or CHECKOUT
 
 RUNNER = r'''
 import sys
@@ -25,7 +29,7 @@ sys.path.insert(0, %(root)r)
 import blues_b200.compat as compat
 compat.install(data_root=%(ref)r)
 import pytest
-sys.exit(pytest.main(['-p', 'no:cacheprovider', '-q', '-rA', '--tb=line', '--rootdir', %(tmp)r, '-c', '/dev/null', %(tmp)r]))
+sys.exit(pytest.main(['-p', 'no:cacheprovider', '-q', '-rA', '--tb=line', '--rootdir', %(tmp)r, '-c', '/dev/null', '--confcutdir', %(tmp)r, %(tmp)r]))
 '''
 
 HOST_ONLY = {
@@ -37,8 +41,6 @@ HOST_ONLY = {
 }
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, 'blues', 'tests')),
-                    reason='reference checkout not mounted (it is absent on the GPU box)')
 def test_reference_test_simulation_runs_unmodified(tmp_path):
     import torch
     if torch.cuda.is_available():
@@ -68,12 +70,10 @@ import blues_b200._native as native
 from tests.oracle_engine import OracleEngine
 native.Engine = OracleEngine            # test infrastructure: the C ABI's Python face answered by the CPU oracle
 import pytest
-sys.exit(pytest.main(['-p', 'no:cacheprovider', '-q', '-rA', '--tb=short', '--rootdir', %(tmp)r, '-c', '/dev/null', %(tmp)r]))
+sys.exit(pytest.main(['-p', 'no:cacheprovider', '-q', '-rA', '--tb=short', '--rootdir', %(tmp)r, '-c', '/dev/null', '--confcutdir', %(tmp)r, %(tmp)r]))
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, 'blues', 'tests')),
-                    reason='reference checkout not mounted (it is absent on the GPU box)')
 def test_reference_tests_pass_on_the_host_layer_over_the_oracle_engine(tmp_path):
     """All 25 tests of ``test_simulation.py`` and ``test_randomrotation.py``, unmodified, against this package's host
     layer (SystemFactory … BLUESSimulation.run, YAML settings, reporters, the rotation move, state sync, accept/reject)
@@ -96,12 +96,16 @@ def test_reference_tests_pass_on_the_host_layer_over_the_oracle_engine(tmp_path)
     assert any('test_randomrotation.py' in p for p in passed)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, 'blues', 'tests')),
-                    reason='reference checkout not mounted (it is absent on the GPU box)')
 def test_fixture_copies_are_verbatim():
-    """tests/golden/reference_checkout/ (input of tests/test_gpu_reference_suite.py) equals the checkout byte for byte."""
-    base = os.path.join(ROOT, 'tests', 'golden', 'reference_checkout', 'blues', 'tests')
-    for rel in ('test_simulation.py', 'test_randomrotation.py', 'test_ethylene.py', 'data/TOL-parm.prmtop', 'data/TOL-parm.inpcrd',
-                'data/ethylene_system.xml', 'data/ethylene_structure.pdb'):
-        with open(os.path.join(base, rel), 'rb') as a, open(os.path.join(REFERENCE, 'blues', 'tests', rel), 'rb') as b:
-            assert a.read() == b.read(), rel
+    """tests/golden/reference_checkout/ (input of tests/test_gpu_reference_suite.py) is unchanged: each file matches the
+    SHA-256 digest recorded for it in tests/golden/reference_checkout_sha256.json.  Where ``BLUES_REFERENCE`` names a
+    checkout, its files must match the same digests, i.e. the copies equal that checkout byte for byte."""
+    with open(os.path.join(ROOT, 'tests', 'golden', 'reference_checkout_sha256.json')) as fh:
+        digests = json.load(fh)
+    assert sorted(digests) == sorted(('test_simulation.py', 'test_randomrotation.py', 'test_ethylene.py',
+                                      'data/TOL-parm.prmtop', 'data/TOL-parm.inpcrd', 'data/ethylene_system.xml',
+                                      'data/ethylene_structure.pdb'))
+    for base in sorted({CHECKOUT, REFERENCE}):
+        for rel, want in digests.items():
+            with open(os.path.join(base, 'blues', 'tests', rel), 'rb') as fh:
+                assert hashlib.sha256(fh.read()).hexdigest() == want, (base, rel)

@@ -41,7 +41,7 @@ def main(argv):
     for name in ('test_simulation.py', 'test_randomrotation.py'):
         shutil.copy(os.path.join(ref, 'blues', 'tests', name), tmp)
     os.chdir(tmp)
-    return pytest.main(['-p', 'no:cacheprovider', '--rootdir', tmp, '-c', '/dev/null', tmp] + args)
+    return pytest.main(['-p', 'no:cacheprovider', '--rootdir', tmp, '-c', '/dev/null', '--confcutdir', tmp, tmp] + args)
 
 
 if __name__ == '__main__':
