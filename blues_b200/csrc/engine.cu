@@ -95,20 +95,14 @@ struct bl_handle {
     std::vector<double> host_tmp;
     double skin = 0.0; int cell_capacity = 0;
     int build_cq = 0, build_ctas = 0;
-    bool builder2 = false; int build2_ctas = 0;  // BLUES_B200_BUILDER=2: ballot-compaction list builder (measured 10 % slower than
-                                                 // the shared-memory sub-list builder, gpurun_out/r2_builder.log: kept for reference)
     bool debug_sync = false, debug_reported = false;   // BLUES_B200_DEBUG_SYNC
     int int_block = 32;          // BLUES_B200_INT_BLOCK: threads per k_integrate CTA (one constraint cluster per thread)
     bool fold_zero = true;       // step programs: force zeroing + rebuild latch inside the INTEGRATE launch before an evaluation
     int spread_split = 0;        // BLUES_B200_SPREAD_SPLIT: y-bands per x-plane of k_pme_spread at <= 2 walkers (0: one wave, see bl_create)
     int spread_threads = 1024;   // BLUES_B200_SPREAD_THREADS: 512 or 1024
-    int pme_cl = 16;             // BLUES_B200_PME_CL: CTAs of the reciprocal-space cluster kernel (8 or 16)
-    int own_dft = 0;             // reciprocal space: 0 cuFFT, 1 three fused direct-DFT kernels, 2 one cluster kernel (small grids)
-    size_t dft_smem = 0;
     int pair_per_sm = 0, n_sm = 148;   // BLUES_B200_PAIR_PER_SM: resident k_pair4 CTAs per SM (0: one CTA per row block)
     int pair_lanes = 8;          // BLUES_B200_PAIR_LANES: lanes per i-atom in k_pair4 (8, 16, 32)
     int pair_x2 = 2;             // BLUES_B200_PAIR_X2: 0 off, 2 / 4 = k_pair4 (packed FFMA2 arithmetic) with that many entries per trip
-    int pair_variant = 132;      // BLUES_B200_PAIR: 0 = k_pair (round 1), else k_pair2 <ewald, lanes, U> (see enqueue_eval); measured: gpurun_out/pair_sweep.log
     int graph_steps = 4;         // plain NCMC steps captured per CUDA graph
     bool pdl = true;             // programmatic dependent launch on the B -> flip -> A -> sort edges (BLUES_B200_PDL=0: off)
     // diagnostic timeline (BLUES_B200_TIMELINE=1): events recorded inside the step graphs, read after every replay
@@ -239,16 +233,20 @@ static void launch_pdl(bl_handle* h, void (*kernel)(KArgs...), dim3 grid, dim3 b
     cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
-template <typename... KArgs, typename... Args>
-static void launch_pdl_smem(bl_handle* h, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = h->pdl ? 1 : 0;
-    cudaLaunchKernelEx(&cfg, kernel, args...);
+// k_pair2 launch of an evaluation that k_pair4 does not take.  PME uses the polynomial Ewald force (EWALD 1) wherever
+// its fit holds (Dev::ewk_ok); reaction field and no-cutoff have no Ewald term.
+template <int METHOD, bool ENERGY>
+static void launch_pair2(const Dev& d, cudaStream_t st, int skip) {
+    const dim3 grid(cdiv((long long)d.Npad * NL_LANES, NL_BLOCK), d.R);
+    if constexpr (METHOD == NB_PME) {
+        if (d.ewk_ok) {
+            if (d.nl_u16) k_pair2<METHOD, ENERGY, unsigned short, 1><<<grid, NL_BLOCK, 0, st>>>(d, skip);
+            else k_pair2<METHOD, ENERGY, int, 1><<<grid, NL_BLOCK, 0, st>>>(d, skip);
+            return;
+        }
+    }
+    if (d.nl_u16) k_pair2<METHOD, ENERGY, unsigned short, 0><<<grid, NL_BLOCK, 0, st>>>(d, skip);
+    else k_pair2<METHOD, ENERGY, int, 0><<<grid, NL_BLOCK, 0, st>>>(d, skip);
 }
 
 // ---- force / energy evaluation at the current positions ---------------------------------------------------
@@ -262,7 +260,7 @@ static void enqueue_eval(bl_handle* h, bool energy, int adv_noise, int adv_md, i
     const int R = d.R, N = d.N;
     // frozen atoms (mass 0): force-only evaluations inside a step program leave their rows out (BLUES_B200_SKIP_FROZEN=0:
     // off).  The forces then cover the mobile atoms only; a host force query re-evaluates in full (forces_partial).
-    const int skip = (in_program && !energy && h->skip_frozen && d.n_frozen > 0 && h->pair_variant > 0) ? 1 : 0;
+    const int skip = (in_program && !energy && h->skip_frozen && d.n_frozen > 0) ? 1 : 0;
     h->forces_partial = skip != 0;
     {
         // latches the rebuild request (unless the integrator did), then (only if due) the cell sort
@@ -300,43 +298,14 @@ static void enqueue_eval(bl_handle* h, bool energy, int adv_noise, int adv_md, i
               else k_pme_spread<512><<<dim3(d.gx, ys, R), 512, sm, s2>>>(d, fcache);
           } else k_pme_spread<256><<<dim3(d.gx, 4, R), 256, (size_t)(d.gy / 4 + 1) * d.gz * sizeof(int) * (fcache ? 2 : 1), s2>>>(d, fcache); }
         tl_mark(h, s2, TL_SPREAD);
-        if (h->own_dft == 2) {
-            // one cluster kernel for the whole transform chain
-            LaunchTimer t(h, BL_K_FFT, s2);
-            const int P = cdiv(d.gx, h->pme_cl);
-            if (h->pme_cl == 16) {
-                if (energy) launch_pdl_smem(h, k_pme_dft_cluster<true, 16>, dim3(16, R), dim3(PME_CL_THREADS), h->dft_smem, s2, d, P);
-                else launch_pdl_smem(h, k_pme_dft_cluster<false, 16>, dim3(16, R), dim3(PME_CL_THREADS), h->dft_smem, s2, d, P);
-            } else {
-                if (energy) launch_pdl_smem(h, k_pme_dft_cluster<true, PME_CL>, dim3(PME_CL, R), dim3(PME_CL_THREADS), h->dft_smem, s2, d, P);
-                else launch_pdl_smem(h, k_pme_dft_cluster<false, PME_CL>, dim3(PME_CL, R), dim3(PME_CL_THREADS), h->dft_smem, s2, d, P);
-            }
-            tl_mark(h, s2, TL_C2R);
-        } else if (h->own_dft) {
-            const int Zc = d.gz / 2 + 1;
-            const size_t sm1 = sizeof(float) * ((d.gy * d.gz + 1) & ~1) + sizeof(float2) * (d.gy * Zc + d.gz + d.gy);
-            const size_t sm3 = sizeof(float2) * (2 * d.gy * Zc + d.gz + d.gy);
-            { LaunchTimer t(h, BL_K_FFT, s2);
-              launch_pdl_smem(h, k_pme_dft_zy, dim3(d.gx, R), dim3(PME_DFT_THREADS), sm1, s2, d); }
-            tl_mark(h, s2, TL_R2C);
-            { LaunchTimer t(h, BL_K_PME_CONVOLVE, s2);
-              const dim3 gridx(cdiv(d.gy * Zc, PME_X_LINES), R);
-              if (energy) launch_pdl_smem(h, k_pme_dft_x<true>, gridx, dim3(PME_X_LINES * 32), 0, s2, d);
-              else launch_pdl_smem(h, k_pme_dft_x<false>, gridx, dim3(PME_X_LINES * 32), 0, s2, d); }
-            tl_mark(h, s2, TL_CONV);
-            { LaunchTimer t(h, BL_K_FFT, s2);
-              launch_pdl_smem(h, k_pme_idft_yz, dim3(d.gx, R), dim3(PME_DFT_THREADS), sm3, s2, d); }
-            tl_mark(h, s2, TL_C2R);
-        } else {
-            { LaunchTimer t(h, BL_K_FFT, s2); cufftExecR2C(h->plan_r2c, d.grid_r, reinterpret_cast<cufftComplex*>(d.grid_c)); }
+        { LaunchTimer t(h, BL_K_FFT, s2); cufftExecR2C(h->plan_r2c, d.grid_r, reinterpret_cast<cufftComplex*>(d.grid_c)); }
         tl_mark(h, s2, TL_R2C);
-            { LaunchTimer t(h, BL_K_PME_CONVOLVE, s2);
-              if (energy) k_pme_convolve<true><<<dim3(cdiv(d.csize, 256), R), 256, 0, s2>>>(d);
-              else k_pme_convolve<false><<<dim3(cdiv(d.csize, 256), R), 256, 0, s2>>>(d); }
-            tl_mark(h, s2, TL_CONV);
+        { LaunchTimer t(h, BL_K_PME_CONVOLVE, s2);
+          if (energy) k_pme_convolve<true><<<dim3(cdiv(d.csize, 256), R), 256, 0, s2>>>(d);
+          else k_pme_convolve<false><<<dim3(cdiv(d.csize, 256), R), 256, 0, s2>>>(d); }
+        tl_mark(h, s2, TL_CONV);
         { LaunchTimer t(h, BL_K_FFT, s2); cufftExecC2R(h->plan_c2r, reinterpret_cast<cufftComplex*>(d.grid_c), d.grid_r); }
         tl_mark(h, s2, TL_C2R);
-        }
         if (!h->profiling) cudaStreamWaitEvent(s2, h->ev_fork2, 0);      // the gather adds to the cleared force accumulators
         { LaunchTimer t(h, BL_K_PME_GATHER, s2);
           if (R <= 2) k_pme_gather5<<<dim3(cdiv(cdiv(N, 6) * 32, 128), R), 128, 0, s2>>>(d, skip);
@@ -401,69 +370,18 @@ static void enqueue_eval(bl_handle* h, bool energy, int adv_noise, int adv_md, i
         LaunchTimer t(h, BL_K_NEIGHBOR);
         dim3 grid(h->build_ctas);                          // persistent single-warp CTAs shared by all walkers
         const size_t smem = build_smem_bytes(h->build_cq, d.nl_u16 ? 2 : 4);
-        if (h->builder2) {
-            dim3 grid2(h->build2_ctas);
-            if (d.nl_u16) k_build_list2<unsigned short><<<grid2, 32, 0, st>>>(d);
-            else k_build_list2<int><<<grid2, 32, 0, st>>>(d);
-        } else if (d.nl_u16) k_build_list<unsigned short><<<grid, 32, smem, st>>>(d, h->build_cq);
+        if (d.nl_u16) k_build_list<unsigned short><<<grid, 32, smem, st>>>(d, h->build_cq);
         else k_build_list<int><<<grid, 32, smem, st>>>(d, h->build_cq);
     }
     tl_mark(h, st, TL_BUILD);
-    if (h->pair_variant >= 1000) {
-        LaunchTimer t(h, BL_K_PAIR);
-        // 1000 + 100 * ewald + 10 * log2(lanes): cp.async ring (k_pair3)
-        const int ew = ((h->pair_variant / 100) % 10) && d.ewk_ok && d.nb_method == 4 ? 1 : 0;
-        const int lanes = 1 << ((h->pair_variant / 10) % 10);
-        dim3 grid(cdiv((long long)d.Npad * lanes, NL_BLOCK), R);
-#define P3C(M, E, T, L, W) k_pair3<M, E, T, L, W><<<grid, NL_BLOCK, 0, st>>>(d)
-#define P3B(M, E, T, L) if (ew) P3C(M, E, T, L, 1); else P3C(M, E, T, L, 0)
-#define P3A(M, E, T) if (lanes == 4) { P3B(M, E, T, 4); } else if (lanes == 16) { P3B(M, E, T, 16); } else { P3B(M, E, T, 8); }
-#define P30(M, E) if (d.nl_u16) { P3A(M, E, unsigned short) } else { P3A(M, E, int) }
-#define P3E(M) if (energy) { P30(M, true) } else { P30(M, false) }
-        if (d.nb_method == 4) { P3E(NB_PME) }
-        else if (d.nb_method == 2) { P3E(NB_RF) }
-        else { P3E(NB_NOCUT) }
-#undef P3C
-#undef P3B
-#undef P3A
-#undef P30
-#undef P3E
-    } else if (use_x2) {
+    if (use_x2) {
         launch_pair4(st, split ? 2 : 0);
         if (split) cudaStreamWaitEvent(st, h->ev_join5, 0);
-    } else if (h->pair_variant > 0) {
-        LaunchTimer t(h, BL_K_PAIR);
-        // variant = 100 * ewald + 10 * log2(lanes) + U  (BLUES_B200_PAIR; 0 = the round-1 kernel)
-        const int ew = (h->pair_variant / 100) && d.ewk_ok && d.nb_method == 4 ? 1 : 0;
-        const int lanes = 1 << ((h->pair_variant / 10) % 10), U = h->pair_variant % 10;
-        dim3 grid(cdiv((long long)d.Npad * lanes, NL_BLOCK), R);
-#define PV3(M, E, T, L, UU, W) k_pair2<M, E, T, L, UU, W><<<grid, NL_BLOCK, 0, st>>>(d, skip)
-#define PV2(M, E, T, L, UU) if (ew) PV3(M, E, T, L, UU, 1); else PV3(M, E, T, L, UU, 0)
-#define PV1(M, E, T) if (lanes == 8 && U == 2) { PV2(M, E, T, 8, 2); } else if (lanes == 8 && U == 4) { PV2(M, E, T, 8, 4); } \
-                     else if (lanes == 16 && U == 2) { PV2(M, E, T, 16, 2); } else if (lanes == 4 && U == 4) { PV2(M, E, T, 4, 4); } \
-                     else { PV2(M, E, T, 16, 4); }
-#define PV0(M, E) if (d.nl_u16) { PV1(M, E, unsigned short) } else { PV1(M, E, int) }
-#define PVE(M) if (energy) { PV0(M, true) } else { PV0(M, false) }
-        if (d.nb_method == 4) { PVE(NB_PME) }
-        else if (d.nb_method == 2) { PVE(NB_RF) }
-        else { PVE(NB_NOCUT) }
-#undef PV3
-#undef PV2
-#undef PV1
-#undef PV0
-#undef PVE
     } else {
         LaunchTimer t(h, BL_K_PAIR);
-        dim3 grid(cdiv((long long)d.Npad * NL_LANES, NL_BLOCK), R);
-#define PAIR2(M, E)                                                           \
-        if (d.nl_u16) k_pair<M, E, unsigned short><<<grid, NL_BLOCK, 0, st>>>(d); \
-        else k_pair<M, E, int><<<grid, NL_BLOCK, 0, st>>>(d)
-#define PAIR(M) if (energy) { PAIR2(M, true); } else { PAIR2(M, false); }
-        if (d.nb_method == 4) { PAIR(NB_PME); }
-        else if (d.nb_method == 2) { PAIR(NB_RF); }
-        else { PAIR(NB_NOCUT); }
-#undef PAIR2
-#undef PAIR
+        if (d.nb_method == NB_PME) { if (energy) launch_pair2<NB_PME, true>(d, st, skip); else launch_pair2<NB_PME, false>(d, st, skip); }
+        else if (d.nb_method == NB_RF) { if (energy) launch_pair2<NB_RF, true>(d, st, skip); else launch_pair2<NB_RF, false>(d, st, skip); }
+        else { if (energy) launch_pair2<NB_NOCUT, true>(d, st, skip); else launch_pair2<NB_NOCUT, false>(d, st, skip); }
     }
     tl_mark(h, st, TL_PAIR);
     if (pme) cudaStreamWaitEvent(st, h->ev_join, 0);
@@ -626,7 +544,7 @@ static void issue(bl_handle* h, const std::vector<Launch>& ls, HostCounters& hc,
             const int prefetch = hc.noise_ready > 0 ? 0 : noise_lookahead(ls, k);
             const bool pre_zeroed = h->fold_zero && k > 0 && !ls[k - 1].is_eval;
             if (!dry) enqueue_eval(h, l.energy, hc.pending_noise, hc.pending_md, l.cm_mode, prefetch, pre_zeroed, true);
-            else h->forces_partial = !l.energy && h->skip_frozen && h->d.n_frozen > 0 && h->pair_variant > 0;
+            else h->forces_partial = !l.energy && h->skip_frozen && h->d.n_frozen > 0;
             if (prefetch > 0) hc.noise_ready = prefetch;
             hc.pending_noise = 0;
             hc.pending_md = 0;
@@ -1002,7 +920,6 @@ int bl_create(const bl_topology* t, int device, int n_replicas, uint64_t seed, b
     cudaDeviceGetAttribute(&h->n_sm, cudaDevAttrMultiProcessorCount, device);
     if (getenv("BLUES_B200_PAIR_LANES")) { const int l = atoi(getenv("BLUES_B200_PAIR_LANES")); h->pair_lanes = l == 16 || l == 32 || l == 4 ? l : 8; }
     if (getenv("BLUES_B200_PAIR_X2")) h->pair_x2 = atoi(getenv("BLUES_B200_PAIR_X2"));
-    if (getenv("BLUES_B200_PAIR")) h->pair_variant = atoi(getenv("BLUES_B200_PAIR"));
     if (getenv("BLUES_B200_DEBUG_SYNC") && atoi(getenv("BLUES_B200_DEBUG_SYNC"))) { h->debug_sync = true; h->use_graphs = false; h->pdl = false; }
     if (getenv("BLUES_B200_SPREAD_SPLIT")) h->spread_split = atoi(getenv("BLUES_B200_SPREAD_SPLIT"));
     if (getenv("BLUES_B200_SPREAD_THREADS")) h->spread_threads = atoi(getenv("BLUES_B200_SPREAD_THREADS")) == 1024 ? 1024 : 512;
@@ -1259,7 +1176,6 @@ int bl_create(const bl_topology* t, int device, int n_replicas, uint64_t seed, b
     d.atom_cell = dalloc<int>(h, RN); d.rank = dalloc<int>(h, RN);
     d.posq_s = dalloc<float4>(h, (size_t)R * d.Npad);
     d.sigeps_s = dalloc<float2>(h, (size_t)R * d.Npad);
-    d.rec_s = dalloc<float4>(h, (size_t)R * d.Npad * 2);
     d.orig_s = dalloc<int>(h, (size_t)R * d.Npad);
     {
         // row capacity per atom: 1.5 x the mean number of atoms inside the list-cutoff sphere (+ margin)
@@ -1301,13 +1217,6 @@ int bl_create(const bl_topology* t, int device, int n_replicas, uint64_t seed, b
         if (R > 2 && per_sm > 2) per_sm -= 1;
         if (getenv("BLUES_B200_BUILD_PER_SM")) per_sm = std::max(1, std::min(per_sm, atoi(getenv("BLUES_B200_BUILD_PER_SM"))));
         h->build_ctas = std::max(32, std::min(R * (cdiv(d.Npad, BUILD_GROUP) + 64), per_sm * n_sm));
-        if (getenv("BLUES_B200_BUILDER")) h->builder2 = atoi(getenv("BLUES_B200_BUILDER")) == 2;
-        int per_sm2 = 0;
-        if (d.nl_u16) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm2, k_build_list2<unsigned short>, 32, 0);
-        else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm2, k_build_list2<int>, 32, 0);
-        per_sm2 = std::max(1, per_sm2);
-        if (R > 2 && per_sm2 > 4) per_sm2 -= 2;          // leave room for the other streams' kernels
-        h->build2_ctas = std::max(32, std::min(R * (cdiv(d.Npad, BUILD_GROUP) + 64), per_sm2 * n_sm));
     }
     // PME
     if (d.pme) {
@@ -1338,48 +1247,6 @@ int bl_create(const bl_topology* t, int device, int n_replicas, uint64_t seed, b
         std::vector<float> mx, my, mz;
         bspline_moduli_host(d.gx, mx); bspline_moduli_host(d.gy, my); bspline_moduli_host(d.gz, mz);
         d.bmod_x = dupload(h, mx); d.bmod_y = dupload(h, my); d.bmod_z = dupload(h, mz);
-        {
-            auto twiddles = [&](int L) {
-                std::vector<float2> tw(L);
-                for (int m = 0; m < L; ++m) tw[m] = make_float2((float)cos(2.0 * M_PI * m / L), (float)sin(2.0 * M_PI * m / L));
-                return dupload(h, tw);
-            };
-            d.tw_x = twiddles(d.gx); d.tw_y = twiddles(d.gy); d.tw_z = twiddles(d.gz);
-            // direct DFTs cost O(points x (X + Y + Z)): they beat cuFFT's seven launches up to ~32 points per dimension
-            // (24 x 25 x 28: 33 us against 45); beyond that cuFFT wins by far (45 x 48 x 54: 264 us against ~40)
-            const int dft_limit = getenv("BLUES_B200_DFT_LIMIT") ? atoi(getenv("BLUES_B200_DFT_LIMIT")) : 32;
-            const bool small = d.gx <= PME_DFT_MAX && d.gy <= PME_DFT_MAX && d.gz <= PME_DFT_MAX &&
-                               d.gx <= dft_limit && d.gy <= dft_limit && d.gz <= dft_limit;
-            // measured again in round 2 (bench.py, same box): cuFFT 7 632 steps/s at one walker and 13 086 walker-steps/s at
-            // eight, the cluster kernel (16 CTAs, packed complex arithmetic) 7 554 and 12 625 — inside the four-stream
-            // evaluation cuFFT's seven small kernels spread over the idle SMs while one cluster waits for sixteen free SMs of
-            // one GPC.  cuFFT (the library call the north star allows) is the default; BLUES_B200_DFT=2 / 1 select the own kernels.
-            h->own_dft = 0;
-            (void)small;
-            if (getenv("BLUES_B200_DFT")) h->own_dft = small ? atoi(getenv("BLUES_B200_DFT")) : 0;
-            {
-                h->pme_cl = getenv("BLUES_B200_PME_CL") ? (atoi(getenv("BLUES_B200_PME_CL")) == 16 ? 16 : PME_CL) : h->pme_cl;
-                if (d.gx < 16) h->pme_cl = PME_CL;
-                const int Zc2 = d.gz / 2 + 1, P = cdiv(d.gx, h->pme_cl);
-                h->dft_smem = sizeof(float4) * (2 * (size_t)d.gy + 2 * d.gx) +
-                              sizeof(float2) * (2 * (size_t)P * d.gy * Zc2 + d.gz + (PME_CL_THREADS / 32) * 2 * d.gx) +
-                              sizeof(float) * ((size_t)P * d.gy * d.gz + 4);
-                if (h->dft_smem > 200 * 1024 && h->own_dft == 2) h->own_dft = 1;
-                raise_dyn_smem(k_pme_dft_cluster<true, PME_CL>, device, h->dft_smem);
-                raise_dyn_smem(k_pme_dft_cluster<false, PME_CL>, device, h->dft_smem);
-                raise_dyn_smem(k_pme_dft_cluster<true, 16>, device, h->dft_smem);
-                raise_dyn_smem(k_pme_dft_cluster<false, 16>, device, h->dft_smem);
-                cudaFuncSetAttribute(k_pme_dft_cluster<true, 16>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-                cudaFuncSetAttribute(k_pme_dft_cluster<false, 16>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-            }
-            const int Zc = d.gz / 2 + 1;
-            const size_t sm = std::max(sizeof(float) * ((d.gy * d.gz + 1) & ~1) + sizeof(float2) * (d.gy * Zc + d.gz + d.gy),
-                                       sizeof(float2) * (2 * d.gy * Zc + d.gz + d.gy));
-            if (h->own_dft && sm > 48 * 1024) {
-                raise_dyn_smem(k_pme_dft_zy, device, sm);
-                raise_dyn_smem(k_pme_idft_yz, device, sm);
-            }
-        }
         int n[3] = {d.gx, d.gy, d.gz};
         if (cufftPlanMany(&h->plan_r2c, 3, n, nullptr, 1, d.gsize, nullptr, 1, d.csize, CUFFT_R2C, R) != CUFFT_SUCCESS ||
             cufftPlanMany(&h->plan_c2r, 3, n, nullptr, 1, d.csize, nullptr, 1, d.gsize, CUFFT_C2R, R) != CUFFT_SUCCESS)

@@ -99,7 +99,6 @@ struct Dev {
     int* group_first; int group_capacity;   // [R][group_capacity] (first sorted index << 4 | atoms) of every build group
     int* rank;                              // [R*N] position of atom a in the sorted order
     float4* posq_s; float2* sigeps_s; int* orig_s;   // [R*Npad] sorted copies (pads: NaN position, orig -1)
-    float4* rec_s;                          // [R*Npad][2] packed sorted records for k_pair3's gathers: (x, y, z, q), (sigma/2, 2 sqrt eps, -, -)
     int nl_M;                               // capacity of one row of the Verlet list
     int* nl_count;                          // [R*Npad]
     void* nl_list;                          // [R*Npad][nl_M] sorted indices of the neighbours within cutoff + skin
@@ -137,7 +136,6 @@ struct Dev {
     int* grid_frozen;                       // [R][gsize], null when nothing is frozen
     int* frozen_grid_state;                 // [R] 0: rebuild in the next spread launch, 1: valid
     float* bmod_x; float* bmod_y; float* bmod_z;
-    float2* tw_x; float2* tw_y; float2* tw_z;       // (cos, sin)(2 pi m / L) of the direct-DFT reciprocal-space kernels
     double self_energy_coeff;               // -k_e alpha/sqrt(pi) sum q^2  (constant)
     double sumq;
     double dispersion_coeff;

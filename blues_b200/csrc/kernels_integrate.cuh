@@ -488,7 +488,7 @@ __device__ __forceinline__ void run_cluster(const Dev& d, const IntegratorConsts
         vel[a] = make_double4(s.v[k][0], s.v[k][1], s.v[k][2], 0.0);
         const float4 pf = wrapped_mirror(d, s.x[k][0], s.x[k][1], s.x[k][2], d.charge[a]);
         d.posq[(size_t)r * N + a] = pf;
-        { const size_t sl = (size_t)r * d.Npad + d.rank[(size_t)r * N + a]; d.posq_s[sl] = pf; d.rec_s[2 * sl] = pf; }
+        { const size_t sl = (size_t)r * d.Npad + d.rank[(size_t)r * N + a]; d.posq_s[sl] = pf; }
         const float4 pr = d.pos_ref[(size_t)r * N + a];
         float ddx = pf.x - pr.x, ddy = pf.y - pr.y, ddz = pf.z - pr.z;
         if (d.periodic) {
@@ -630,7 +630,7 @@ __device__ __forceinline__ void run_cluster_generic(const Dev& d, const Integrat
         vel[a] = make_double4(s.v[k][0], s.v[k][1], s.v[k][2], 0.0);
         const float4 pf = wrapped_mirror(d, s.x[k][0], s.x[k][1], s.x[k][2], d.charge[a]);
         d.posq[(size_t)r * N + a] = pf;
-        { const size_t sl = (size_t)r * d.Npad + d.rank[(size_t)r * N + a]; d.posq_s[sl] = pf; d.rec_s[2 * sl] = pf; }
+        { const size_t sl = (size_t)r * d.Npad + d.rank[(size_t)r * N + a]; d.posq_s[sl] = pf; }
         const float4 pr = d.pos_ref[(size_t)r * N + a];
         float ddx = pf.x - pr.x, ddy = pf.y - pr.y, ddz = pf.z - pr.z;
         if (d.periodic) {
@@ -798,7 +798,7 @@ __global__ void k_refresh_mirrors(Dev d, int request_rebuild, int clear_replica)
     const double4 p = d.pos[(size_t)r * d.N + a];
     const float4 pf = wrapped_mirror(d, p.x, p.y, p.z, d.charge[a]);
     d.posq[(size_t)r * d.N + a] = pf;
-    { const size_t sl = (size_t)r * d.Npad + d.rank[(size_t)r * d.N + a]; d.posq_s[sl] = pf; d.rec_s[2 * sl] = pf; }
+    { const size_t sl = (size_t)r * d.Npad + d.rank[(size_t)r * d.N + a]; d.posq_s[sl] = pf; }
     if (a == 0 && request_rebuild) { d.g[r].rebuild_request = 2; d.g[r].prune_request = 1; }
 }
 

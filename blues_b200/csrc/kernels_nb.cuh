@@ -1,7 +1,6 @@
 // Neighbour-list construction (K1) and the tiled direct-space pair kernel (K2).
 #pragma once
 #include <cooperative_groups.h>
-#include <type_traits>
 #include "engine.cuh"
 
 // ---------------------------------------------------------------------------------------------------------
@@ -167,8 +166,6 @@ __global__ void __cluster_dims__(SORT_CTAS, 1, 1) __launch_bounds__(1024) k_sort
         posq_s[s] = p;
         sigeps_s[s] = se;
         d.mobile_s[(size_t)r * Npad + s] = d.invmass[a] > 0.0 ? 1 : 0;
-        d.rec_s[2 * ((size_t)r * Npad + s)] = p;
-        d.rec_s[2 * ((size_t)r * Npad + s) + 1] = make_float4(se.x, se.y, 0.f, 0.f);
         pos_ref[a] = p;
     }
     const float qnan = __int_as_float(0x7fc00000);
@@ -176,8 +173,6 @@ __global__ void __cluster_dims__(SORT_CTAS, 1, 1) __launch_bounds__(1024) k_sort
         posq_s[s] = make_float4(qnan, qnan, qnan, 0.f);
         sigeps_s[s] = make_float2(0.f, 0.f);
         d.mobile_s[(size_t)r * Npad + s] = 0;
-        d.rec_s[2 * ((size_t)r * Npad + s)] = make_float4(qnan, qnan, qnan, 0.f);
-        d.rec_s[2 * ((size_t)r * Npad + s) + 1] = make_float4(0.f, 0.f, 0.f, 0.f);
         orig_s[s] = -1;
     }
     if (tid == 0) {
@@ -559,192 +554,7 @@ __global__ void __launch_bounds__(32) k_build_list(Dev d, int cq) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// k_build_list2: the same Verlet rows by warp-ballot compaction (round 2).  One warp per group of <= 8 cell-sorted atoms
-// as before, but lane = CANDIDATE: the 32 candidates of a chunk sit one per lane in registers, the (<= 8) group atoms
-// are broadcast from shared memory, so a chunk costs 8 x (1 LDS + ~9 ALU) warp-instructions for 256 distance tests
-// instead of 8 per-lane tests against staged candidates; chunks whose candidates all lie farther than the list cutoff
-// from the group's bounding box are skipped after one point-to-box test; survivors of atom a are ranked with
-// __ballot_sync / __popc and stored straight into its row (consecutive lanes -> consecutive entries).  No shared-memory
-// sub-lists, no flush pass; scan order and therefore row order are fixed (reproducible sums downstream).
-// ---------------------------------------------------------------------------------------------------------
-struct BuildGroupSmem {
-    float4 runs[BUILD_MAX_RUNS];
-    int off[BUILD_MAX_RUNS + 4];
-    float4 gat[BUILD_GROUP];            // group atoms: x, y, z, topology index (bits); NaN position for idle slots
-    ull gwin[BUILD_GROUP];
-    int2 gspan[BUILD_GROUP];            // exclusion window of every group atom as [first topology index, width]
-    unsigned char gfar[BUILD_GROUP];
-};
-
-template <bool RINT, typename IDX>
-__device__ __forceinline__ void build_stream2(const Dev& d, const float4* __restrict__ posq_s, const int* __restrict__ orig_s,
-                                              BuildGroupSmem& sm, int nruns, bool rx, bool ry, bool rz, int lane, bool anyfar,
-                                              float lox, float hix, float loy, float hiy, float loz, float hiz,
-                                              int (&cnt)[BUILD_GROUP], IDX* rows) {
-    const float cut2 = d.list_cutoff2;
-    const float bx = d.boxf[0], by = d.boxf[1], bz = d.boxf[2], ibx = d.boxf[3], iby = d.boxf[4], ibz = d.boxf[5];
-    const float qnan = __int_as_float(0x7fc00000);
-    const int nl_M = d.nl_M;
-    const int total = sm.off[nruns];
-    const unsigned int lt = (1u << lane) - 1u;
-    // centre and half extent of the group's bounding box (point-to-box distance of a candidate)
-    const float cx = 0.5f * (lox + hix), cy = 0.5f * (loy + hiy), cz = 0.5f * (loz + hiz);
-    const float ex = 0.5f * (hix - lox), ey = 0.5f * (hiy - loy), ez = 0.5f * (hiz - loz);
-    int kp = 0;
-    float4 cnext = make_float4(qnan, qnan, qnan, 0.f);
-    int ojnext = 0;
-    auto fetch = [&](int c) {
-        cnext = make_float4(qnan, qnan, qnan, 0.f);
-        if (c < total) {
-            while (c >= sm.off[kp + 1]) ++kp;
-            const float4 rn = sm.runs[kp];
-            const int s = __float_as_int(rn.w) + (c - sm.off[kp]);
-            const float4 p = posq_s[s];
-            ojnext = orig_s[s];
-            cnext = make_float4(p.x + rn.x, p.y + rn.y, p.z + rn.z, __int_as_float(s));   // shifted image; w = sorted index
-        }
-    };
-    fetch(lane);
-    for (int c0 = 0; c0 < total; c0 += 32) {
-        const float4 c = cnext;
-        const int oj = ojnext;
-        fetch(c0 + 32 + lane);
-        // distance from the candidate to the group's bounding box: a lower bound of its distance to every group atom
-        {
-            float qx = c.x - cx, qy = c.y - cy, qz = c.z - cz;
-            if (RINT) {
-                if (rx) qx -= bx * rintf(qx * ibx);
-                if (ry) qy -= by * rintf(qy * iby);
-                if (rz) qz -= bz * rintf(qz * ibz);
-            }
-            qx = fmaxf(fabsf(qx) - ex, 0.f); qy = fmaxf(fabsf(qy) - ey, 0.f); qz = fmaxf(fabsf(qz) - ez, 0.f);
-            if (!__any_sync(0xffffffffu, qx * qx + qy * qy + qz * qz < cut2)) continue;      // NaN (padding) compares false
-        }
-        bool near = false;
-#pragma unroll
-        for (int k = 0; k < BUILD_GROUP; ++k) { const int2 sp = sm.gspan[k]; near = near || (unsigned int)(oj - sp.x) <= (unsigned int)sp.y; }
-        const bool check = anyfar || __any_sync(0xffffffffu, near);
-        unsigned int bits = 0;
-#pragma unroll
-        for (int a = 0; a < BUILD_GROUP; ++a) {
-            const float4 g = sm.gat[a];
-            float dx = c.x - g.x, dy = c.y - g.y, dz = c.z - g.z;
-            if (RINT) {
-                if (rx) dx -= bx * rintf(dx * ibx);
-                if (ry) dy -= by * rintf(dy * iby);
-                if (rz) dz -= bz * rintf(dz * ibz);
-            }
-            bits |= (dx * dx + dy * dy + dz * dz < cut2) ? (1u << a) : 0u;
-        }
-        if (check && bits) {
-            // rare: this chunk holds a candidate inside the exclusion window of a group atom (or far exclusions exist)
-            for (int a = 0; a < BUILD_GROUP; ++a) {
-                if (!((bits >> a) & 1u)) continue;
-                const int oi = __float_as_int(sm.gat[a].w);
-                const unsigned int dd = (unsigned int)(oj - oi + 32);
-                bool ok = true;
-                if (dd < 64u) ok = !((sm.gwin[a] >> dd) & 1ull);                 // includes the atom itself (bit 32)
-                else if (sm.gfar[a]) ok = !pair_excluded(d, oi, sm.gwin[a], true, oj, d.has_far[oj]);
-                if (!ok) bits &= ~(1u << a);
-            }
-        }
-        const int sj = __float_as_int(c.w);
-#pragma unroll
-        for (int a = 0; a < BUILD_GROUP; ++a) {
-            const bool mine = (bits >> a) & 1u;
-            const unsigned int m = __ballot_sync(0xffffffffu, mine);
-            if (m) {
-                const int pos = cnt[a] + __popc(m & lt);
-                if (mine && pos < nl_M) rows[(size_t)a * nl_M + pos] = (IDX)sj;
-                cnt[a] += __popc(m);
-            }
-        }
-    }
-}
-
-template <typename IDX>
-__global__ void __launch_bounds__(32, 24) k_build_list2(Dev d) {
-    __shared__ BuildGroupSmem sm;
-    const int lane = threadIdx.x;
-    const int N = d.N, Npad = d.Npad;
-    for (int wk = 0; wk < d.R; ++wk) {
-    const int r = (blockIdx.x + wk) % d.R;
-    Globals& g = d.g[r];
-    if (!g.do_rebuild) continue;
-    const float4* __restrict__ posq_s = d.posq_s + (size_t)r * Npad;
-    const int* __restrict__ orig_s = d.orig_s + (size_t)r * Npad;
-    const int* __restrict__ start = d.cell_start + (size_t)r * (d.ncells + 1);
-    const int* __restrict__ groups = d.group_first + (size_t)r * d.group_capacity;
-    const int n_groups = g.n_groups;
-    const int a = lane & (BUILD_GROUP - 1);
-    for (;;) {
-        int gi = 0;
-        if (lane == 0) gi = atomicAdd(&g.build_cursor, 1);
-        gi = __shfl_sync(0xffffffffu, gi, 0);
-        if (gi >= n_groups) break;
-        const int packed = groups[gi];
-        const int i0 = packed >> 4, na = packed & 15;
-        const bool valid = a < na;
-        const int i = valid ? i0 + a : i0;
-        const float qnan = __int_as_float(0x7fc00000);
-        const float4 pa = posq_s[i];
-        const int oi = orig_s[i];
-        const ull wi = valid ? (d.excl_win[oi] | (1ull << 32)) : 0ull;
-        const bool fari = valid ? d.has_far[oi] : false;
-        const bool anyfar = __any_sync(0xffffffffu, fari);
-        __syncwarp();                                   // the previous group's readers are done with the shared tables
-        if (lane < BUILD_GROUP) {
-            sm.gat[lane] = valid ? make_float4(pa.x, pa.y, pa.z, __int_as_float(oi)) : make_float4(qnan, qnan, qnan, __int_as_float(-1));
-            sm.gwin[lane] = wi;
-            sm.gfar[lane] = fari ? 1 : 0;
-            // idle slots: an empty window ([1, 0] never contains a candidate)
-            const int below = valid ? 32 - (__ffsll((long long)wi) - 1) : 0, above = valid ? 31 - __clzll((long long)wi) : 0;
-            sm.gspan[lane] = valid ? make_int2(oi - below, below + above) : make_int2(0x7fffffff, 0);
-        }
-        int cnt[BUILD_GROUP];
-#pragma unroll
-        for (int k = 0; k < BUILD_GROUP; ++k) cnt[k] = 0;
-        IDX* rows = reinterpret_cast<IDX*>(d.nl_list) + ((size_t)r * Npad + i0) * d.nl_M;
-        if (!d.periodic) {
-            if (lane == 0) { sm.runs[0] = make_float4(0.f, 0.f, 0.f, __int_as_float(0)); sm.off[0] = 0; sm.off[1] = N; }
-            __syncwarp();
-            build_stream2<false, IDX>(d, posq_s, orig_s, sm, 1, false, false, false, lane, anyfar, -3.0e38f, 3.0e38f,
-                                      -3.0e38f, 3.0e38f, -3.0e38f, 3.0e38f, cnt, rows);
-        } else {
-            const int ncx = d.ncell[0], ncy = d.ncell[1], ncz = d.ncell[2];
-            int cx, cy, cz;
-            atom_cell_coords(d, pa, cx, cy, cz);
-            const int xa = __reduce_min_sync(0xffffffffu, cx), xb = __reduce_max_sync(0xffffffffu, cx);
-            const int ya = __reduce_min_sync(0xffffffffu, cy), yb = __reduce_max_sync(0xffffffffu, cy);
-            const int za = __reduce_min_sync(0xffffffffu, cz), zb = __reduce_max_sync(0xffffffffu, cz);
-            const float lox = warp_min(pa.x), hix = warp_max(pa.x), loy = warp_min(pa.y), hiy = warp_max(pa.y);
-            const float loz = warp_min(pa.z), hiz = warp_max(pa.z);
-            const bool rx = xb - xa + 5 > ncx, ry = yb - ya + 5 > ncy, rz = zb - za + 2 * d.zreach + 1 > ncz;
-            const int x0 = rx ? 0 : xa - 2, x1 = rx ? ncx - 1 : xb + 2;
-            const int y0 = ry ? 0 : ya - 2, y1 = ry ? ncy - 1 : yb + 2;
-            const int nruns = build_group_runs(d, start, lane, rx, ry, rz, x0, x1, y0, y1, za, zb, lox, hix, loy, hiy, loz,
-                                               hiz, sm.runs, sm.off);
-            if (rx || ry || rz)
-                build_stream2<true, IDX>(d, posq_s, orig_s, sm, nruns, rx, ry, rz, lane, anyfar, lox, hix, loy, hiy,
-                                         loz, hiz, cnt, rows);
-            else
-                build_stream2<false, IDX>(d, posq_s, orig_s, sm, nruns, false, false, false, lane, anyfar, lox, hix,
-                                          loy, hiy, loz, hiz, cnt, rows);
-        }
-        int mycnt = 0;
-#pragma unroll
-        for (int k = 0; k < BUILD_GROUP; ++k) mycnt = (lane == k) ? cnt[k] : mycnt;
-        if (__any_sync(0xffffffffu, lane < na && mycnt > d.nl_M)) { if (lane == 0) g.item_overflow = 1; }
-        if (lane < na) d.nl_count[(size_t)r * Npad + i0 + lane] = min(mycnt, d.nl_M);
-    }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// k_pair: direct-space Lennard-Jones + Coulomb (Ewald erfc / reaction field / plain) over the Verlet list.
-// NL_LANES lanes share one i-atom (register resident) and stride over its neighbour list with coalesced index
-// loads; j data are gathered from the spatially sorted float4 mirror (L1/L2 resident); the partial forces are
-// combined by warp shuffles in a fixed order and leave the warp as 64-bit fixed-point atomics.
+// Direct-space pair kernels: Lennard-Jones + Coulomb (Ewald erfc / reaction field / plain) over the Verlet list.
 // ---------------------------------------------------------------------------------------------------------
 #define NB_NOCUT 0
 #define NB_RF 2
@@ -760,95 +570,18 @@ __device__ __forceinline__ float erfc_times(float ar, float expar) {
 // same result): the XU pipe, which also serves rsqrt / rcp / ex2, is the busiest execution unit of the pair loop
 __device__ __forceinline__ float rint_fma(float x) { return __fadd_rn(__fadd_rn(x, 12582912.0f), -12582912.0f); }
 
-template <int METHOD, bool ENERGY, typename IDX>
-__global__ void __launch_bounds__(NL_BLOCK) k_pair(Dev d) {
-    const int r = blockIdx.y;
-    const int lane = threadIdx.x & 31;
-    const int part = lane & (NL_LANES - 1);
-    const int i = (blockIdx.x * NL_BLOCK + threadIdx.x) / NL_LANES;
-    const int N = d.N, Npad = d.Npad;
-    if (i >= Npad) return;
-    const float4* __restrict__ posq_s = d.posq_s + (size_t)r * Npad;
-    const float2* __restrict__ sigeps_s = d.sigeps_s + (size_t)r * Npad;
-    const IDX* __restrict__ list = reinterpret_cast<const IDX*>(d.nl_list) + ((size_t)r * Npad + i) * d.nl_M;
-    const int cnt = d.nl_count[(size_t)r * Npad + i];
-    const float bx = d.boxf[0], by = d.boxf[1], bz = d.boxf[2];
-    const float ibx = d.boxf[3], iby = d.boxf[4], ibz = d.boxf[5];
-    const float cut2 = METHOD == NB_NOCUT ? 3.0e38f : d.cutoff2;
-    const float alpha = d.alpha, krf = d.krf, crf = d.crf;
-    const float4 pi = posq_s[i];
-    const float2 se_i = sigeps_s[i];
-    const float qi = pi.w * (float)ONE_4PI_EPS0;
-    float fx = 0.f, fy = 0.f, fz = 0.f, etot = 0.f;
-#pragma unroll 4
-    for (int k = part; k < cnt; k += NL_LANES) {
-        const int s = (int)list[k];
-        const float4 pj = posq_s[s];
-        const float2 se_j = sigeps_s[s];
-        float dx = pi.x - pj.x, dy = pi.y - pj.y, dz = pi.z - pj.z;
-        if (METHOD != NB_NOCUT) {
-            dx -= bx * rint_fma(dx * ibx);
-            dy -= by * rint_fma(dy * iby);
-            dz -= bz * rint_fma(dz * ibz);
-        }
-        const float r2 = dx * dx + dy * dy + dz * dz;
-        // branch-free: entries in the skin shell are computed and masked, so the loads of the unrolled iterations
-        // are issued together instead of behind a divergent branch
-        const float in = r2 < cut2 ? 1.0f : 0.0f;
-        const float invr = rsqrtf(r2);
-        const float invr2 = invr * invr;
-        const float sig = se_i.x + se_j.x;
-        const float s2 = sig * sig * invr2;
-        const float s6 = s2 * s2 * s2;
-        const float eps4 = se_i.y * se_j.y * in;
-        float de = eps4 * (12.0f * s6 * s6 - 6.0f * s6);
-        const float qq = qi * pj.w * in;
-        if (METHOD == NB_PME) {
-            const float ar = alpha * r2 * invr;
-            const float ex = __expf(-ar * ar);
-            const float ec = erfc_times(ar, ex);
-            de += qq * invr * (ec + (float)TWO_OVER_SQRT_PI * ar * ex);
-            if (ENERGY) etot += eps4 * (s6 * s6 - s6) + qq * invr * ec;
-        } else if (METHOD == NB_RF) {
-            de += qq * (invr - 2.0f * krf * r2);
-            if (ENERGY) etot += eps4 * (s6 * s6 - s6) + qq * (invr + krf * r2 - crf) ;
-        } else {
-            de += qq * invr;
-            if (ENERGY) etot += eps4 * (s6 * s6 - s6) + qq * invr;
-        }
-        de *= invr2;
-        fx += dx * de; fy += dy * de; fz += dz * de;
-    }
-    // combine the NL_LANES partial sums (fixed xor tree → deterministic)
-#pragma unroll
-    for (int o = NL_LANES / 2; o > 0; o >>= 1) {
-        fx += __shfl_xor_sync(0xffffffffu, fx, o);
-        fy += __shfl_xor_sync(0xffffffffu, fy, o);
-        fz += __shfl_xor_sync(0xffffffffu, fz, o);
-    }
-    if (part == 0 && i < N) {
-        const int oi = d.orig_s[(size_t)r * Npad + i];
-        long long* fenv = d.f_env + (size_t)r * 3 * N;
-        fx_addf(&fenv[oi], fx, (float)FORCE_SCALE);
-        fx_addf(&fenv[N + oi], fy, (float)FORCE_SCALE);
-        fx_addf(&fenv[2 * N + oi], fz, (float)FORCE_SCALE);
-    }
-    if (ENERGY) {
-        // every pair appears in both atoms' lists
-        const float e = warp_sum(etot);
-        if (lane == 0 && e != 0.f) fx_add(&d.eacc[r * N_ETERMS + E_PAIR], 0.5 * (double)e, ENERGY_SCALE);
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------------
-// k_pair2: the same sum as k_pair, software pipelined.  ncu on k_pair (profiles/r01_final2_ncu_summary.md, source page):
-// 67 % of the stall samples are long-scoreboard waits at the two consumers of a dependent load chain — the list index,
-// then the gather it addresses.  Here a lane owns the entries part, part + LANES, ... of its atom's row and works in
-// trips of U entries: while trip t is computed the gathers of trip t + 1 and the index loads of trip t + 2 are in flight.
+// k_pair2: the pair sum of energy evaluations, and of force-only evaluations that k_pair4 does not cover.  NL_LANES
+// lanes share one i-atom (register resident); a lane owns the entries part, part + NL_LANES, ... of the atom's row and
+// works in trips of U = 2 entries, software pipelined: while trip t is computed the gathers of trip t + 1 and the
+// index loads of trip t + 2 are in flight.  Without the pipeline, 67 % of the stall samples were long-scoreboard waits
+// at the two consumers of a dependent load chain — the list index, then the gather it addresses
+// (profiles/r01_final2_ncu_summary.md, source page).  j data are gathered from the cell-sorted mirrors; the partial
+// forces are combined by warp shuffles in a fixed order and leave the warp as 64-bit fixed-point atomics.
 // Reads may run up to two trips past the end of a row: rows are contiguous (the next row holds valid indices) and the
 // array carries that much slack after the last row; such entries are masked by their position in the row.
 // EWALD 1: real-space Ewald force from the polynomial of Dev::ewk (no MUFU.EX2 / MUFU.RCP: the XU pipe is the busiest
-// unit of k_pair); energies, on the steps that need them, still come from erfc.
+// unit of the pair loop); energies, on the steps that need them, still come from erfc.
 // ---------------------------------------------------------------------------------------------------------
 #define PAIR_SLACK_ENTRIES 512
 // volatile so that the loads of the NEXT trips keep their place at the top of the loop body (the compiler otherwise
@@ -933,8 +666,9 @@ __device__ __forceinline__ void pair_trip(const Dev& d, const float4 (&pc)[U], c
     }
 }
 
-template <int METHOD, bool ENERGY, typename IDX, int LANES, int U, int EWALD>
+template <int METHOD, bool ENERGY, typename IDX, int EWALD>
 __global__ void __launch_bounds__(NL_BLOCK) k_pair2(Dev d, int skip_frozen) {
+    constexpr int LANES = NL_LANES, U = 2;
     const int r = blockIdx.y;
     const int lane = threadIdx.x & 31;
     const int part = lane & (LANES - 1);
@@ -993,6 +727,7 @@ __global__ void __launch_bounds__(NL_BLOCK) k_pair2(Dev d, int skip_frozen) {
         fx_addf(&fenv[2 * N + oi], fz, (float)FORCE_SCALE);
     }
     if (ENERGY) {
+        // every pair appears in both atoms' lists
         const float e = warp_sum(etot);
         if (lane == 0 && e != 0.f) fx_add(&d.eacc[r * N_ETERMS + E_PAIR], 0.5 * (double)e, ENERGY_SCALE);
     }
@@ -1136,127 +871,6 @@ __global__ void PAIR4_BOUNDS k_pair4(Dev d, int skip_frozen, int phase) {
         fx_addf(&fenv[N + oi], fy, (float)FORCE_SCALE);
         fx_addf(&fenv[2 * N + oi], fz, (float)FORCE_SCALE);
     }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// k_pair3: the pair sum with asynchronous gathers (cp.async → shared memory ring).  ptxas schedules plain loads next to
-// their consumers whatever the source order (k_pair2's software pipeline ends up with every load at the bottom of the loop
-// body), so the prefetch is made explicit: a lane owns the entry PAIRS (2 part, 2 part + 1) + 2 LANES m of its atom's row.
-// In iteration t it waits for the copy group of trip t, reads the two indices of trip t + 2 from its index slot, issues
-// the gathers of trip t + 2 (posq 16 B, sigeps 8 B per entry) and the index copy of trip t + 4 as one group, then computes
-// trip t from shared memory while two groups are in flight.  Every thread touches only its own slots: no barrier.
-// ---------------------------------------------------------------------------------------------------------
-#define P3_STAGES 3
-__device__ __forceinline__ void cp_async16(unsigned int dst, const void* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async8(unsigned int dst, const void* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async4(unsigned int dst, const void* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-template <typename IDX> __device__ __forceinline__ void p3_copy_idx(unsigned int dst, const IDX* src);
-template <> __device__ __forceinline__ void p3_copy_idx<unsigned short>(unsigned int dst, const unsigned short* src) { cp_async4(dst, src); }
-template <> __device__ __forceinline__ void p3_copy_idx<int>(unsigned int dst, const int* src) { cp_async8(dst, src); }
-
-template <int METHOD, bool ENERGY, typename IDX, int LANES, int EWALD>
-__global__ void __launch_bounds__(NL_BLOCK) k_pair3(Dev d) {
-    // per thread and stage: 2 records of 2 x float4 and 2 indices; arrays are [stage][slot][thread] (conflict-free LDS.128)
-    __shared__ float4 s_rec[P3_STAGES * 4 * NL_BLOCK];
-    __shared__ IDX s_idx[P3_STAGES * 2 * NL_BLOCK];           // [stage][thread][2]
-    const int r = blockIdx.y;
-    const int tid = threadIdx.x;
-    const int lane = tid & 31;
-    const int part = lane & (LANES - 1);
-    const int i = (blockIdx.x * NL_BLOCK + tid) / LANES;
-    const int N = d.N, Npad = d.Npad;
-    if (i >= Npad) return;
-    const float4* __restrict__ rec = d.rec_s + 2 * (size_t)r * Npad;
-    const IDX* __restrict__ lp = reinterpret_cast<const IDX*>(d.nl_list) + ((size_t)r * Npad + i) * d.nl_M + 2 * part;
-    const int cnt = d.nl_count[(size_t)r * Npad + i];
-    const int ntrip = (cnt + 2 * LANES - 1) / (2 * LANES);       // the same for the LANES lanes of an atom
-    const float cut2 = METHOD == NB_NOCUT ? 3.0e38f : d.cutoff2;
-    const float4 pi = rec[2 * i];
-    const float4 ri = rec[2 * i + 1];
-    const float2 se_i = make_float2(ri.x, ri.y);
-    const float qi = pi.w * (float)ONE_4PI_EPS0;
-    float fx = 0.f, fy = 0.f, fz = 0.f, etot = 0.f;
-    const unsigned int a_rec = (unsigned int)__cvta_generic_to_shared(s_rec) + tid * 16u;
-    const unsigned int a_idx = (unsigned int)__cvta_generic_to_shared(s_idx) + tid * 2u * (unsigned int)sizeof(IDX);
-    constexpr unsigned int REC_STAGE = 4 * NL_BLOCK * 16, REC_SLOT = NL_BLOCK * 16, IDX_STAGE = 2 * NL_BLOCK * sizeof(IDX);
-    constexpr int TRIP = 2 * LANES;                              // entries of a row consumed per trip
-    auto gather = [&](int stage, int s0, int s1) {
-        const float4* g0 = rec + 2 * s0;
-        const float4* g1 = rec + 2 * s1;
-        cp_async16(a_rec + stage * REC_STAGE, g0);
-        cp_async16(a_rec + stage * REC_STAGE + REC_SLOT, g0 + 1);
-        cp_async16(a_rec + stage * REC_STAGE + 2 * REC_SLOT, g1);
-        cp_async16(a_rec + stage * REC_STAGE + 3 * REC_SLOT, g1 + 1);
-    };
-    // one iteration with compile-time stage numbers: trip t lives in stage ST, trip t + 2 goes to ST2, the indices of
-    // trip t + 4 to the slot trip t + 1 used
-    auto step = [&](int t, auto st_c, auto st2_c, auto st4_c) {
-        constexpr int ST = decltype(st_c)::value, ST2 = decltype(st2_c)::value, ST4 = decltype(st4_c)::value;
-        cp_async_wait<1>();                  // gathers of trip t and the indices of trip t + 2 have landed
-        {
-            const IDX* si = s_idx + ST2 * 2 * NL_BLOCK + tid * 2;
-            int s0, s1;
-            if (sizeof(IDX) == 2) {
-                const unsigned int v = *reinterpret_cast<const unsigned int*>(si);
-                s0 = (int)(v & 0xffffu); s1 = (int)(v >> 16);
-            } else {
-                const int2 v = *reinterpret_cast<const int2*>(si);
-                s0 = v.x; s1 = v.y;
-            }
-            gather(ST2, s0, s1);
-            p3_copy_idx<IDX>(a_idx + ST4 * IDX_STAGE, lp + (t + 4) * TRIP);
-            cp_async_commit();
-        }
-        float4 pc[2];
-        float2 ec[2];
-        const float4 q0 = s_rec[(ST * 4 + 1) * NL_BLOCK + tid], q1 = s_rec[(ST * 4 + 3) * NL_BLOCK + tid];
-        pc[0] = s_rec[(ST * 4 + 0) * NL_BLOCK + tid]; pc[1] = s_rec[(ST * 4 + 2) * NL_BLOCK + tid];
-        ec[0] = make_float2(q0.x, q0.y); ec[1] = make_float2(q1.x, q1.y);
-        pair_trip<METHOD, ENERGY, 2, EWALD>(d, pc, ec, 2 * part + TRIP * t, cnt, pi, se_i, qi, cut2, fx, fy, fz, etot);
-    };
-    // prologue: trips 0 and 1 need their indices in registers; the index copies of trips 2 and 3 ride in the same groups
-    {
-        const int s00 = (int)lp[0], s01 = (int)lp[1], s10 = (int)lp[TRIP], s11 = (int)lp[TRIP + 1];
-        gather(0, s00, s01);
-        p3_copy_idx<IDX>(a_idx + 2 * IDX_STAGE, lp + 2 * TRIP);
-        cp_async_commit();
-        gather(1, s10, s11);
-        p3_copy_idx<IDX>(a_idx + 0 * IDX_STAGE, lp + 3 * TRIP);
-        cp_async_commit();
-    }
-    using I0 = std::integral_constant<int, 0>; using I1 = std::integral_constant<int, 1>; using I2 = std::integral_constant<int, 2>;
-    for (int t = 0; t < ntrip; t += 3) {
-        step(t, I0(), I2(), I1());
-        if (t + 1 < ntrip) step(t + 1, I1(), I0(), I2());
-        if (t + 2 < ntrip) step(t + 2, I2(), I1(), I0());
-    }
-    cp_async_wait<0>();
-#pragma unroll
-    for (int o = LANES / 2; o > 0; o >>= 1) {
-        fx += __shfl_xor_sync(0xffffffffu, fx, o);
-        fy += __shfl_xor_sync(0xffffffffu, fy, o);
-        fz += __shfl_xor_sync(0xffffffffu, fz, o);
-    }
-    if (part == 0 && i < N) {
-        const int oi = d.orig_s[(size_t)r * Npad + i];
-        long long* fenv = d.f_env + (size_t)r * 3 * N;
-        fx_addf(&fenv[oi], fx, (float)FORCE_SCALE);
-        fx_addf(&fenv[N + oi], fy, (float)FORCE_SCALE);
-        fx_addf(&fenv[2 * N + oi], fz, (float)FORCE_SCALE);
-    }
-    if (ENERGY) {
-        const float e = warp_sum(etot);
-        if (lane == 0 && e != 0.f) fx_add(&d.eacc[r * N_ETERMS + E_PAIR], 0.5 * (double)e, ENERGY_SCALE);
     }
 }
 

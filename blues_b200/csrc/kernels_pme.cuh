@@ -208,343 +208,6 @@ __global__ void __launch_bounds__(256) k_pme_convolve(Dev d) {
     }
 }
 
-// ---------------------------------------------------------------------------------------------------------
-// Reciprocal space without cuFFT for small grids (every dimension <= PME_DFT_MAX): three kernels instead of seven.
-// The grids of the measured systems (24 x 25 x 28, 24^3) are so small that a library FFT is pure launch latency — six
-// kernels of ~6 us each around the convolution, 3-4 x longer while the pair kernel shares the SMs
-// (profiles/r01_step_timeline.md).  A direct DFT per dimension with exact twiddle tables costs 4.5 MFMA for
-// 24 x 25 x 28, nothing for the device, and lets the passes fuse:
-//   k_pme_dft_zy   one CTA per x-plane: real z-transform (half spectrum), y-transform        -> grid_c
-//   k_pme_dft_x    CTAs of lines along x: x-transform, influence function (+ energy), inverse x-transform (in place)
-//   k_pme_idft_yz  one CTA per x-plane: inverse y-transform, Hermitian inverse z-transform   -> grid_r
-// Conventions are cuFFT's (unnormalised, forward sign -), so spread / gather and the energy are unchanged.
-// ---------------------------------------------------------------------------------------------------------
-#define PME_DFT_MAX 64
-#define PME_DFT_THREADS 256
-
-// out = sum_n in[n * stride] * w^(sign k n), w = exp(-2 pi i / L), twiddles tw[m] = (cos, sin)(2 pi m / L)
-__device__ __forceinline__ float2 dft_line_c(const float2* in, int stride, int L, int k, const float2* tw, float sign) {
-    float re = 0.f, im = 0.f;
-    int m = 0;
-    for (int n = 0; n < L; ++n) {
-        const float2 v = in[n * stride];
-        const float2 w = tw[m];
-        const float ws = sign * w.y;                 // forward: e^{-i theta} = (cos, -sin)
-        re = fmaf(v.x, w.x, re); re = fmaf(-v.y, ws, re);
-        im = fmaf(v.x, ws, im); im = fmaf(v.y, w.x, im);
-        m += k; m -= m >= L ? L : 0;
-    }
-    return make_float2(re, im);
-}
-
-__global__ void __launch_bounds__(PME_DFT_THREADS) k_pme_dft_zy(Dev d) {
-    extern __shared__ float s_dft[];                 // plane [Y][Z] floats, then tmp [Y][Zc] float2, then twiddles
-    cudaGridDependencySynchronize();
-    const int r = blockIdx.y, x = blockIdx.x;
-    const int Y = d.gy, Z = d.gz, Zc = Z / 2 + 1;
-    float* plane = s_dft;
-    float2* tmp = reinterpret_cast<float2*>(s_dft + ((Y * Z + 1) & ~1));
-    float2* twz = tmp + Y * Zc;
-    float2* twy = twz + Z;
-    const float* src = d.grid_r + (size_t)r * d.gsize + (size_t)x * Y * Z;
-    for (int k = threadIdx.x; k < Y * Z; k += blockDim.x) plane[k] = src[k];
-    for (int k = threadIdx.x; k < Z; k += blockDim.x) twz[k] = d.tw_z[k];
-    for (int k = threadIdx.x; k < Y; k += blockDim.x) twy[k] = d.tw_y[k];
-    __syncthreads();
-    for (int o = threadIdx.x; o < Y * Zc; o += blockDim.x) {
-        const int y = o / Zc, kz = o - y * Zc;
-        const float* in = plane + y * Z;
-        float re = 0.f, im = 0.f;
-        int m = 0;
-        for (int z = 0; z < Z; ++z) {
-            const float v = in[z];
-            const float2 w = twz[m];
-            re = fmaf(v, w.x, re); im = fmaf(-v, w.y, im);
-            m += kz; m -= m >= Z ? Z : 0;
-        }
-        tmp[o] = make_float2(re, im);
-    }
-    __syncthreads();
-    float2* dst = d.grid_c + (size_t)r * d.csize + (size_t)x * Y * Zc;
-    for (int o = threadIdx.x; o < Y * Zc; o += blockDim.x) {
-        const int ky = o / Zc, kz = o - ky * Zc;
-        dst[o] = dft_line_c(tmp + kz, Zc, Y, ky, twy, -1.f);
-    }
-}
-
-// lines along x: PME_X_LINES consecutive (ky, kz) lines per CTA, one thread per (line, kx)
-#define PME_X_LINES 8
-template <bool ENERGY>
-__global__ void __launch_bounds__(PME_X_LINES * 32) k_pme_dft_x(Dev d) {
-    __shared__ float2 s_line[PME_X_LINES][PME_DFT_MAX + 1];
-    __shared__ float2 s_out[PME_X_LINES][PME_DFT_MAX + 1];
-    __shared__ float2 s_tw[PME_DFT_MAX];
-    cudaGridDependencySynchronize();
-    const int r = blockIdx.y;
-    const int X = d.gx, Y = d.gy, Zc = d.gz / 2 + 1, plane = Y * Zc;
-    const int li = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int line = blockIdx.x * PME_X_LINES + li;              // = ky * Zc + kz
-    const bool live = line < plane;
-    float2* grid = d.grid_c + (size_t)r * d.csize;
-    for (int k = threadIdx.x; k < X; k += blockDim.x) s_tw[k] = d.tw_x[k];
-    if (live)
-        for (int x = lane; x < X; x += 32) s_line[li][x] = grid[(size_t)x * plane + line];
-    __syncthreads();
-    double e = 0.0;
-    if (live) {
-        const int ky = line / Zc, kz = line - ky * Zc;
-        const int my = ky <= Y / 2 ? ky : ky - Y;
-        const float fy = my * d.boxf[4], fz = kz * d.boxf[5];
-        const float V = d.boxf[0] * d.boxf[1] * d.boxf[2];
-        const float pi2_over_a2 = 9.8696044010893586f / (d.alpha * d.alpha);
-        for (int kx = lane; kx < X; kx += 32) {
-            float2 c = dft_line_c(&s_line[li][0], 1, X, kx, s_tw, -1.f);
-            float eterm = 0.f;
-            if (kx != 0 || line != 0) {
-                const int mx = kx <= X / 2 ? kx : kx - X;
-                const float fx = mx * d.boxf[3];
-                const float m2 = fx * fx + fy * fy + fz * fz;
-                const float denom = m2 * d.bmod_x[kx] * d.bmod_y[ky] * d.bmod_z[kz] * 3.14159265358979f * V;
-                eterm = (float)ONE_4PI_EPS0 * expf(-pi2_over_a2 * m2) / denom;
-            }
-            if (ENERGY) {
-                const double w = (kz == 0 || (2 * kz == d.gz)) ? 1.0 : 2.0;
-                e += 0.5 * w * (double)eterm * ((double)c.x * c.x + (double)c.y * c.y);
-            }
-            s_out[li][kx] = make_float2(c.x * eterm, c.y * eterm);
-        }
-    }
-    __syncthreads();
-    if (live)
-        for (int x = lane; x < X; x += 32) grid[(size_t)x * plane + line] = dft_line_c(&s_out[li][0], 1, X, x, s_tw, 1.f);
-    if (ENERGY) {
-        e = warp_sum(e);
-        if (lane == 0 && e != 0.0) fx_add(&d.eacc[r * N_ETERMS + E_PME], e, ENERGY_SCALE);
-    }
-}
-
-__global__ void __launch_bounds__(PME_DFT_THREADS) k_pme_idft_yz(Dev d) {
-    extern __shared__ float s_dft[];                 // in [Y][Zc] float2, tmp [Y][Zc] float2, twiddles
-    cudaGridDependencySynchronize();
-    const int r = blockIdx.y, x = blockIdx.x;
-    const int Y = d.gy, Z = d.gz, Zc = Z / 2 + 1;
-    float2* in = reinterpret_cast<float2*>(s_dft);
-    float2* tmp = in + Y * Zc;
-    float2* twz = tmp + Y * Zc;
-    float2* twy = twz + Z;
-    const float2* src = d.grid_c + (size_t)r * d.csize + (size_t)x * Y * Zc;
-    for (int k = threadIdx.x; k < Y * Zc; k += blockDim.x) in[k] = src[k];
-    for (int k = threadIdx.x; k < Z; k += blockDim.x) twz[k] = d.tw_z[k];
-    for (int k = threadIdx.x; k < Y; k += blockDim.x) twy[k] = d.tw_y[k];
-    __syncthreads();
-    for (int o = threadIdx.x; o < Y * Zc; o += blockDim.x) {
-        const int y = o / Zc, kz = o - y * Zc;
-        tmp[o] = dft_line_c(in + kz, Zc, Y, y, twy, 1.f);
-    }
-    __syncthreads();
-    float* dst = d.grid_r + (size_t)r * d.gsize + (size_t)x * Y * Z;
-    const bool even = (Z & 1) == 0;
-    for (int o = threadIdx.x; o < Y * Z; o += blockDim.x) {
-        const int y = o / Z, z = o - y * Z;
-        const float2* c = tmp + y * Zc;
-        // Hermitian half spectrum: kz = 0 (and Z / 2 for even Z) count once with their real part, the others twice
-        float acc = c[0].x;
-        int m = z;                                    // (kz z) mod Z for kz = 1
-        const int last = even ? Zc - 1 : Zc;
-        for (int kz = 1; kz < last; ++kz) {
-            const float2 w = twz[m];
-            acc = fmaf(2.f * c[kz].x, w.x, acc);
-            acc = fmaf(-2.f * c[kz].y, w.y, acc);
-            m += z; m -= m >= Z ? Z : 0;
-        }
-        if (even) acc += (z & 1) ? -c[Zc - 1].x : c[Zc - 1].x;
-        dst[o] = acc;
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// k_pme_dft_cluster: the whole reciprocal-space transform chain — forward z, y, x, influence function (+ energy), inverse
-// x, y, z — as ONE kernel on one thread-block cluster per walker.  The timeline (gpurun_out/r2_timeline.log) shows why:
-// while the pair kernel fills the SMs each of the short transform kernels is stretched 4 x (k_pme_dft_zy 10 -> 43 us) and
-// every kernel boundary adds a launch + dependency gap, so the chain, not the pair kernel, is the critical path of the
-// ~5 of 6 steps without a list rebuild.  Here CTA c of the cluster owns the x-planes c P .. c P + P - 1 in shared memory
-// (P = ceil(X / PME_CL)); the z and y passes are local, the x pass reads the lines through distributed shared memory
-// (one warp per (ky, kz) line, staged locally), applies the influence function, transforms back and returns the line to
-// its owners; two cluster barriers in total, no global round trip between the passes.
-// ---------------------------------------------------------------------------------------------------------
-#define PME_CL 8
-#define PME_CL_THREADS 768
-// CL: CTAs of the cluster — 8 (portable) or 16 (B200 allows it with cudaFuncAttributeNonPortableClusterSizeAllowed): the kernel
-// is instruction bound on the SMs of its one cluster (ncu: 864 k warp instructions on 8 SMs, 47 % issue), twice the SMs
-// halve the lines and planes per CTA.  The planes a CTA owns are transformed together (one barrier per pass, not per plane),
-// the complex multiply-adds are packed FP32 pairs (re, im) against twiddle quadruples (c, -s, s, c) / (c, s, -s, c).
-__device__ __forceinline__ unsigned long long pme_pack(float lo, float hi) {
-    unsigned long long r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-    return r;
-}
-__device__ __forceinline__ unsigned long long pme_fma2(unsigned long long a, unsigned long long b, unsigned long long c) {
-    unsigned long long r;
-    asm("fma.rn.ftz.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
-// out = sum_n in[n * stride] * w^(+-k n); tq[m] = (c, -s, s, c) for the forward sign, (c, s, -s, c) for the inverse
-__device__ __forceinline__ float2 dft_line_q(const float2* in, int stride, int L, int k, const float4* tq) {
-    unsigned long long acc0 = pme_pack(0.f, 0.f), acc1 = acc0;          // two chains: even / odd terms
-    int m = 0;
-    int n = 0;
-    for (; n + 1 < L; n += 2) {
-        const float2 v0 = in[n * stride];
-        const float4 t0 = tq[m];
-        m += k; m -= m >= L ? L : 0;
-        const float2 v1 = in[(n + 1) * stride];
-        const float4 t1 = tq[m];
-        m += k; m -= m >= L ? L : 0;
-        acc0 = pme_fma2(pme_pack(v0.x, v0.x), pme_pack(t0.x, t0.y), acc0);
-        acc1 = pme_fma2(pme_pack(v1.x, v1.x), pme_pack(t1.x, t1.y), acc1);
-        acc0 = pme_fma2(pme_pack(v0.y, v0.y), pme_pack(t0.z, t0.w), acc0);
-        acc1 = pme_fma2(pme_pack(v1.y, v1.y), pme_pack(t1.z, t1.w), acc1);
-    }
-    if (n < L) {
-        const float2 v0 = in[n * stride];
-        const float4 t0 = tq[m];
-        acc0 = pme_fma2(pme_pack(v0.x, v0.x), pme_pack(t0.x, t0.y), acc0);
-        acc0 = pme_fma2(pme_pack(v0.y, v0.y), pme_pack(t0.z, t0.w), acc0);
-    }
-    float r0, i0, r1, i1;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(r0), "=f"(i0) : "l"(acc0));
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(r1), "=f"(i1) : "l"(acc1));
-    return make_float2(r0 + r1, i0 + i1);
-}
-
-template <bool ENERGY, int CL>
-__global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(PME_CL_THREADS) k_pme_dft_cluster(Dev d, int P) {
-    namespace cg = cooperative_groups;
-    extern __shared__ float s_dft[];
-    cudaGridDependencySynchronize();
-    cg::cluster_group cluster = cg::this_cluster();
-    const int rank = (int)cluster.block_rank();
-    const int r = blockIdx.y;
-    const int X = d.gx, Y = d.gy, Z = d.gz, Zc = Z / 2 + 1, YZc = Y * Zc, YZ = Y * Z;
-    // shared layout (float4-aligned pieces first): twiddle quadruples fwd / inv for y, x and fwd for z | cplane [P][Y][Zc] float2 |
-    // tmp [P][Y][Zc] float2 | twz (c, s) float2 [Z] | line staging [warps][2][X] float2 | rplane [P][Y][Z] float
-    float4* tqyf = reinterpret_cast<float4*>(s_dft);
-    float4* tqyi = tqyf + Y;
-    float4* tqxf = tqyi + Y;
-    float4* tqxi = tqxf + X;
-    float2* cplane = reinterpret_cast<float2*>(tqxi + X);
-    float2* tmp = cplane + (size_t)P * YZc;
-    float2* twz = tmp + (size_t)P * YZc;
-    float2* sline = twz + Z;                                   // [warps][2][X]
-    float* rplane = reinterpret_cast<float*>(sline + (size_t)(PME_CL_THREADS / 32) * 2 * X);
-    const int tid = threadIdx.x, nt = blockDim.x;
-    for (int k = tid; k < Z; k += nt) twz[k] = d.tw_z[k];
-    for (int k = tid; k < Y; k += nt) { const float2 w = d.tw_y[k]; tqyf[k] = make_float4(w.x, -w.y, w.y, w.x); tqyi[k] = make_float4(w.x, w.y, -w.y, w.x); }
-    for (int k = tid; k < X; k += nt) { const float2 w = d.tw_x[k]; tqxf[k] = make_float4(w.x, -w.y, w.y, w.x); tqxi[k] = make_float4(w.x, w.y, -w.y, w.x); }
-    const int x_first = rank * P;
-    const int np = max(0, min(P, X - x_first));                // planes this CTA owns (the last ranks may own none)
-    // ---- forward z and y passes on all owned planes at once (they are contiguous in the x-major grid)
-    {
-        const float* src = d.grid_r + (size_t)r * d.gsize + (size_t)x_first * YZ;
-        for (int k = tid; k < np * YZ; k += nt) rplane[k] = src[k];
-    }
-    __syncthreads();
-    for (int o = tid; o < np * YZc; o += nt) {
-        const int pl = o / YZc, oo = o - pl * YZc;
-        const int y = oo / Zc, kz = oo - y * Zc;
-        const float* in = rplane + pl * YZ + y * Z;
-        unsigned long long acc = pme_pack(0.f, 0.f);
-        int m = 0;
-        for (int z = 0; z < Z; ++z) {
-            const float v = in[z];
-            const float2 w = twz[m];
-            acc = pme_fma2(pme_pack(v, v), pme_pack(w.x, -w.y), acc);
-            m += kz; m -= m >= Z ? Z : 0;
-        }
-        float re, im;
-        asm("mov.b64 {%0, %1}, %2;" : "=f"(re), "=f"(im) : "l"(acc));
-        tmp[o] = make_float2(re, im);
-    }
-    __syncthreads();
-    for (int o = tid; o < np * YZc; o += nt) {
-        const int pl = o / YZc, oo = o - pl * YZc;
-        const int ky = oo / Zc, kz = oo - ky * Zc;
-        cplane[o] = dft_line_q(tmp + pl * YZc + kz, Zc, Y, ky, tqyf);
-    }
-    cluster.sync();
-    // ---- x pass: line l = ky Zc + kz is handled by CTA l mod CL, one warp per line
-    {
-        const int warp = tid >> 5, lane = tid & 31, nwarps = nt >> 5;
-        float2* lin = sline + (size_t)warp * 2 * X;
-        float2* lout = lin + X;
-        const float V = d.boxf[0] * d.boxf[1] * d.boxf[2];
-        const float pi2_over_a2 = 9.8696044010893586f / (d.alpha * d.alpha);
-        double e = 0.0;
-        for (int l = rank + CL * warp; l < YZc; l += CL * nwarps) {
-            for (int x = lane; x < X; x += 32) {
-                const float2* owner = cluster.map_shared_rank(cplane, x / P);
-                lin[x] = owner[(size_t)(x % P) * YZc + l];
-            }
-            __syncwarp();
-            const int ky = l / Zc, kz = l - ky * Zc;
-            const int my = ky <= Y / 2 ? ky : ky - Y;
-            const float fy = my * d.boxf[4], fz = kz * d.boxf[5];
-            for (int kx = lane; kx < X; kx += 32) {
-                float2 c = dft_line_q(lin, 1, X, kx, tqxf);
-                float eterm = 0.f;
-                if (kx != 0 || l != 0) {
-                    const int mx = kx <= X / 2 ? kx : kx - X;
-                    const float fx = mx * d.boxf[3];
-                    const float m2 = fx * fx + fy * fy + fz * fz;
-                    const float denom = m2 * d.bmod_x[kx] * d.bmod_y[ky] * d.bmod_z[kz] * 3.14159265358979f * V;
-                    eterm = (float)ONE_4PI_EPS0 * expf(-pi2_over_a2 * m2) / denom;
-                }
-                if (ENERGY) {
-                    const double w = (kz == 0 || (2 * kz == Z)) ? 1.0 : 2.0;
-                    e += 0.5 * w * (double)eterm * ((double)c.x * c.x + (double)c.y * c.y);
-                }
-                lout[kx] = make_float2(c.x * eterm, c.y * eterm);
-            }
-            __syncwarp();
-            for (int x = lane; x < X; x += 32) {
-                float2* owner = cluster.map_shared_rank(cplane, x / P);
-                owner[(size_t)(x % P) * YZc + l] = dft_line_q(lout, 1, X, x, tqxi);
-            }
-            __syncwarp();
-        }
-        if (ENERGY) {
-            e = warp_sum(e);
-            if (lane == 0 && e != 0.0) fx_add(&d.eacc[r * N_ETERMS + E_PME], e, ENERGY_SCALE);
-        }
-    }
-    cluster.sync();
-    // ---- inverse y and z passes, real grid back to global memory
-    const bool even = (Z & 1) == 0;
-    for (int o = tid; o < np * YZc; o += nt) {
-        const int pl = o / YZc, oo = o - pl * YZc;
-        const int y = oo / Zc, kz = oo - y * Zc;
-        tmp[o] = dft_line_q(cplane + pl * YZc + kz, Zc, Y, y, tqyi);
-    }
-    __syncthreads();
-    float* dst = d.grid_r + (size_t)r * d.gsize + (size_t)x_first * YZ;
-    for (int o = tid; o < np * YZ; o += nt) {
-        const int pl = o / YZ, oo = o - pl * YZ;
-        const int y = oo / Z, z = oo - y * Z;
-        const float2* c = tmp + pl * YZc + y * Zc;
-        float acc = c[0].x;
-        int m = z;
-        const int last = even ? Zc - 1 : Zc;
-        for (int kz = 1; kz < last; ++kz) {
-            const float2 w = twz[m];
-            acc = fmaf(2.f * c[kz].x, w.x, acc);
-            acc = fmaf(-2.f * c[kz].y, w.y, acc);
-            m += z; m -= m >= Z ? Z : 0;
-        }
-        if (even) acc += (z & 1) ? -c[Zc - 1].x : c[Zc - 1].x;
-        dst[o] = acc;
-    }
-}
-
 // skip_frozen: forces on atoms of mass 0 are not needed (an evaluation inside the integrator program; blues/simulation.py:
 // 364-480 freezes by zeroing masses).  The first thread also marks the frozen share of the charge grid as stored — the
 // whole spread launch that wrote it has finished by the time any gather thread runs.

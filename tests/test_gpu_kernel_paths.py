@@ -476,13 +476,13 @@ def test_reaction_field_neighbour_and_exclusion_sets(R, case):
 
 # ---- E. run-time kernel switches ---------------------------------------------------------------------------------
 
-SWITCHES = ([('PAIR', v) for v in ('0', '124', '1132')] + [('PAIR_X2', v) for v in ('0', '4')] +
-            [('PAIR_LANES', v) for v in ('4', '16', '32')] +
-            [('BUILDER', '2'), ('ZFINE', '1'), ('INT_BLOCK', '64'), ('FOLD_ZERO', '0'), ('GRAPH_STEPS', '1'),
-             ('PDL', '0'), ('DFT', '1'), ('DFT', '2')])
+SWITCHES = ([('PAIR_X2', v) for v in ('0', '4')] + [('PAIR_LANES', v) for v in ('4', '16', '32')] +
+            [('ZFINE', '1'), ('INT_BLOCK', '64'), ('FOLD_ZERO', '0'), ('GRAPH_STEPS', '1'), ('PDL', '0'),
+             ('SKIN', '0.05'), ('BUILD_CQ', '16'), ('BUILD_PER_SM', '1'), ('PAIR_PER_SM', '1'), ('SPREAD_THREADS', '512'),
+             ('NO_PRIORITY', '1')])
 SWITCH_CASES = ([(var, val, 'wat_divaline', (1, 3)) for var, val in SWITCHES] +
                 [('PAIR_SPLIT', '1', 'wat_divaline', (8,))] +
-                [('DFT', v, 'small_grid', (1, 3)) for v in ('1', '2')])
+                [(var, val, 'small_grid', (1, 3)) for var, val in (('SPREAD_SPLIT', '2'), ('SPREAD_THREADS', '512'))])
 
 
 @pytest.mark.gpu
